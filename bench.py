@@ -64,7 +64,13 @@ def parse():
     ap.add_argument("--mp-mode", default="pipelined", choices=["pipelined", "weak"],
                     help="N > 1: 'pipelined' (default) = the 4096^2 problem slab-decomposed, --rhs right-hand sides per GPU sent through "
                          "the slabs one behind the other; 'weak' = only the single-right-hand-side weak-scaling case (n = 4096 sqrt(N))")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="one GPU: after the timed steps, write what the last timed GMRES batch "
+                    "returned as float64 .npy files in DIR: u (right-hand side, sampled point, re/im: every solution at the same "
+                    "seeded sample of at most 48 MB in all), residuals (right-hand side, inner iteration) and info")
+    a = ap.parse_args()
+    if a.dump_outputs and (a.impl != "b200" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs: the b200 arm on one GPU only")
+    return a
 
 
 def workload(args, world, n=None):
@@ -287,6 +293,22 @@ def timed_region(torch, fn):
     return e0.elapsed_time(e1) / 1e3, r
 
 
+def dump_outputs(torch, out_dir, res):
+    """gmres_batch's [(u, info, hist), ...] as float64 .npy files; a larger u is sampled at points fixed by a seed, so that
+    two builds run with the same arguments can be compared output for output"""
+    N, R = res[0][0].numel(), len(res)
+    S = min(N, (48 << 20) // (16 * R))
+    idx = np.arange(N) if S == N else np.sort(np.random.default_rng(0).choice(N, S, replace=False))
+    idx = torch.from_numpy(idx).to(res[0][0].device)
+    hist = np.full((R, max(len(h) for _, _, h in res)), np.nan)
+    for i, (_, _, h) in enumerate(res):
+        hist[i, :len(h)] = h
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "u.npy"), torch.view_as_real(torch.stack([u[idx] for u, _, _ in res])).cpu().numpy())
+    np.save(os.path.join(out_dir, "residuals.npy"), hist)
+    np.save(os.path.join(out_dir, "info.npy"), np.array([info for _, info, _ in res], dtype=np.float64))
+
+
 def true_residual(torch, s, f, u):
     r = s.matvec(u)
     return (torch.linalg.norm(f - r) / torch.linalg.norm(f)).item()
@@ -401,6 +423,8 @@ def run_b200(args):
     bw_ms, bw_n, bw_b = C.c_double(), C.c_int(), C.c_int64()
     lib.hp_profile_read(s.handle, C.byref(bw_ms), C.byref(bw_n), C.byref(bw_b))
     lib.hp_profile_enable(s.handle, 0)
+    if args.dump_outputs:
+        dump_outputs(torch, args.dump_outputs, res)
     # ---- end to end through the public API with host buffers: pinned f -> device, K iterations, u -> host
 
     def e2e():

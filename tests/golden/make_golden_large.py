@@ -26,7 +26,9 @@ Part (D)
 
 Full fields are too large to commit (16 MB each at 1023^2), so a field u[j, i] is stored as: a few full rows, the
 checksum of every row with a fixed random vector z (u @ z), the checksum of every column (z2 @ u), and its norm.
+No committed file exceeds 1 MB: a fixture larger than that is split into <name>.npz, <name>.2.npz, ... (write / load).
 """
+import glob
 import os
 import sys
 import time
@@ -103,10 +105,39 @@ def x_rand(n):
     return rng.standard_normal(n * n) + 1j * rng.standard_normal(n * n)
 
 
+PART_BYTES = 900_000
+
+
+def write(path, out):
+    """np.savez_compressed of the arrays of `out`, in order, spread over path, path[:-4] + '.2.npz', ... so that no file
+    holds more than PART_BYTES of array data"""
+    for old in glob.glob(glob.escape(path[:-4]) + ".[0-9]*.npz"):
+        os.remove(old)
+    parts, size = [{}], 0
+    for k, v in out.items():
+        nb = np.asarray(v).nbytes
+        if parts[-1] and size + nb > PART_BYTES:
+            parts.append({})
+            size = 0
+        parts[-1][k] = v
+        size += nb
+    for i, arrays in enumerate(parts):
+        np.savez_compressed(path if i == 0 else f"{path[:-4]}.{i + 1}.npz", **arrays)
+
+
+def load(path):
+    """the arrays of a fixture written by write(), as one dict"""
+    out, i = dict(np.load(path)), 2
+    while os.path.exists(f"{path[:-4]}.{i}.npz"):
+        out.update(np.load(f"{path[:-4]}.{i}.npz"))
+        i += 1
+    return out
+
+
 def save(case, part, out):
     p = CASES[case]
     name = f"large_n{p['n']}_b{p['b']}_{p['model']}__{part}.npz"
-    np.savez_compressed(os.path.join(HERE, name), **out)
+    write(os.path.join(HERE, name), out)
     print("written", name, {k: getattr(v, "shape", v) for k, v in out.items() if not k.endswith(("_rows", "sum"))}, flush=True)
 
 

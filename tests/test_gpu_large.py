@@ -15,6 +15,7 @@ torch = pytest.importorskip("torch")
 pytestmark = pytest.mark.gpu
 
 from oracle import helmholtz_oracle as orc  # noqa: E402
+from tests.golden.make_golden_large import load as load_fixture  # noqa: E402
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
 MF_TOL = 1e-12          # north_star: preconditioned residuals within 1e-12 relative
@@ -95,7 +96,7 @@ def solver_for(hp, g, front):
 def test_precond_and_operator_vs_reference(hp, path):
     """algo2_4 (code.py:356-385) and A x against the UNMODIFIED reference at n = 63, 511, 1023, 1024 (b = 20), and the
     oracle's paper-diagonal / coupled-front variants on the same inputs."""
-    g = np.load(path)
+    g = load_fixture(path)
     n = int(g["n"])
     omega, c_mat, f_mat = case_fields(hp, g)
     f, xr = dev(f_mat.ravel()), dev(x_rand(n))
@@ -118,7 +119,7 @@ def test_precond_and_operator_vs_reference(hp, path):
 def test_precond_4096_vs_oracle(hp, path):
     """M f and M x_rand at BASELINE's 4096^2 layered configuration against the oracle (SuperLU strip by strip): the error
     accumulated over the chain of 4084 strips, twice."""
-    g = np.load(path)
+    g = load_fixture(path)
     n = int(g["n"])
     omega, c_mat, f_mat = case_fields(hp, g)
     f, xr = dev(f_mat.ravel()), dev(x_rand(n))
@@ -135,7 +136,7 @@ def test_precond_4096_vs_oracle(hp, path):
 def test_gmres_to_convergence(hp, path):
     """GMRES(20), rtol 1e-3, M applied to the vector it is given: iteration count +-1, exit code, history and solution
     against the oracle's run to convergence (diag = reference does not converge and is capped)."""
-    g = np.load(path)
+    g = load_fixture(path)
     n, b = int(g["n"]), int(g["b"])
     diag, front, cap = str(g["diag"]), str(g["front"]), int(g["maxiter"])
     omega, c_mat, f_mat = case_fields(hp, g)

@@ -56,6 +56,7 @@ SIGNATURES = {
     "hp_front_end": (_i, [_vp, _vp, _vp]),
     "hp_precond_apply": (_i, [_vp, _vp, _vp, _i, _vp]),
     "hp_multi_max": (_i, [_vp]),
+    "hp_multi_kernel": (_i, [_vp, _i]),
     "hp_sweep_forward_multi": (_i, [_vp, _i, C.POINTER(_vp), _i, _i, _vp]),
     "hp_sweep_backward_multi": (_i, [_vp, _i, C.POINTER(_vp), _i, _i, _i, _vp]),
     "hp_precond_apply_multi": (_i, [_vp, _i, C.POINTER(_vp), C.POINTER(_vp), _i, _vp]),

@@ -427,10 +427,19 @@ int hp_sweep_launch(hp_solver* s, int mode, cplx* u, const cplx* vin, cplx* yout
     return 0;
 }
 
+// kernel that one launch carrying R right-hand sides runs with the layout of this solver: 2 = hp_sweep4d (tensor cores,
+// R = 8), 1 = hp_sweep4m, 0 = none (the right-hand sides go through the single-vector kernel one by one)
+extern "C" int hp_multi_kernel(hp_solver* s, int R) {
+    if (!s || !s->packets || R < 1 || R > HP_RMAX) return 0;
+    if (R == 8 && !hp_sweep4d_supported(s)) return 2;
+    return hp_sweep4m_supported(s, R) ? 0 : 1;
+}
+
 int hp_sweep_launch_multi(hp_solver* s, int mode, int R, cplx* const* um, int m_from, int m_to, int diag_mode, cudaStream_t st) {
     if (!s->packets) { hp_set_error("sweep: preconditioner not set up"); return 1; }
-    const bool tensor = R == 8 && !hp_sweep4d_supported(s);
-    if (R < 1 || R > HP_RMAX || (!tensor && hp_sweep4m_supported(s, R))) { hp_set_error("sweep: %d right-hand sides per launch not supported by this layout", R); return 1; }
+    const int kernel = hp_multi_kernel(s, R);
+    if (!kernel) { hp_set_error("sweep: %d right-hand sides per launch not supported by this layout", R); return 1; }
+    const bool tensor = kernel == 2;
     int lo = mode == 1 ? m_to : m_from, hi = mode == 1 ? m_from : m_to;
     if (lo > hi) return 0;
     if (lo < s->m_lo || hi > s->m_hi) {

@@ -62,8 +62,8 @@ __device__ __forceinline__ void xload(const cplx* p, unsigned long long& lo, uns
 __device__ __forceinline__ bool xvalid(unsigned long long lo, unsigned long long hi) { return lo != HP_SENTINEL && hi != HP_SENTINEL; }
 // a runaway wait: stop this launch (flag [0]) and leave a mark that survives it (flag [1], read by hp_sweep_status)
 __device__ __forceinline__ void hp_raise_abort(unsigned int* abort_flag) {
+    atomicExch(abort_flag, 1u);
     atomicExch(abort_flag + 1, 1u);
-    hp_raise_abort(abort_flag);
 }
 // spin until the word is valid; on a runaway spin raise the abort flag (the kernel then terminates)
 __device__ __forceinline__ cplx xget(const cplx* p, unsigned int* abort_flag) {

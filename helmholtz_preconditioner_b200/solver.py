@@ -11,7 +11,6 @@ PyTorch is used for device buffers and streams only; every n^2-sized operation i
 There is no CPU path: without the library or a CUDA device these functions raise.
 """
 import ctypes as C
-import os
 import time
 from dataclasses import dataclass, field
 
@@ -246,10 +245,15 @@ class HelmholtzSolver:
             g *= 2
         return g
 
+    def multi_kernel(self, R):
+        """sweep kernel of one launch carrying R right-hand sides: 2 = hp_sweep4d (tensor cores, R = 8), 1 = hp_sweep4m,
+        0 = none (this layout cannot carry R per launch)"""
+        return int(self.lib.hp_multi_kernel(self.handle, int(R)))
+
     def batch_kernel_name(self, R):
         g = self.batch_group(R)
         if g > 1:
-            return "hp_sweep4d_kernel (FP64 tensor cores, 8 right-hand sides)" if g == 8 and not os.environ.get("HP_NO_DMMA") else "hp_sweep4m_kernel"
+            return "hp_sweep4d_kernel (FP64 tensor cores, 8 right-hand sides)" if self.multi_kernel(g) == 2 else "hp_sweep4m_kernel"
         return "hp_sweep4_kernel" if self.layout()["colN"] else "hp_sweep2_kernel"
 
     @staticmethod

@@ -119,6 +119,9 @@ int hp_precond_apply(hp_solver* s, const double* f_dev, double* u_dev, int diag_
  * 1, 2, 4 or 8 and <= hp_multi_max(s) (1 when the partition of the strips does not fit the multi-vector kernel).  Per
  * right-hand side the result equals hp_sweep_forward / hp_sweep_backward / hp_precond_apply up to rounding. */
 int hp_multi_max(hp_solver* s);
+/* Kernel that one launch carrying R right-hand sides runs (the choice hp_sweep_forward_multi / hp_sweep_backward_multi
+ * make): 2 = hp_sweep4d (FP64 tensor cores, R = 8), 1 = hp_sweep4m, 0 = none (R is not supported by this layout). */
+int hp_multi_kernel(hp_solver* s, int R);
 int hp_sweep_forward_multi(hp_solver* s, int R, double* const* u_devs, int m_from, int m_to, void* stream);
 int hp_sweep_backward_multi(hp_solver* s, int R, double* const* u_devs, int m_from, int m_to, int diag_mode, void* stream);
 int hp_precond_apply_multi(hp_solver* s, int R, const double* const* f_devs, double* const* u_devs, int diag_mode, void* stream);

@@ -68,3 +68,27 @@ def test_product_does_not_import_oracle():
             if f.endswith((".py", ".cu", ".cuh", ".h")):
                 txt = open(os.path.join(dirpath, f)).read()
                 assert "import oracle" not in txt and "from oracle" not in txt and "helmholtz_oracle" not in txt, f
+
+
+def test_sweep_abort_raises_both_flags(tmp_path):
+    """hp_raise_abort (csrc/hp_sweep_common.cuh), which a sweep CTA calls when its wait for exchange data runs into
+    HP_SPIN_LIMIT, must store the per-launch flag that stops the other CTAs and the sticky flag that hp_sweep_status
+    reports, and return.  Compiled for sm_100a: straight-line code with exactly two atomic exchanges and no call (a
+    function that calls itself compiles to a CALL into an endless loop, and the stalled sweep would then never end)."""
+    import shutil
+    import subprocess
+    cuda_bin = os.path.join(os.environ.get("CUDA_HOME", "/usr/local/cuda"), "bin")
+    nvcc = shutil.which("nvcc") or shutil.which("nvcc", path=cuda_bin)
+    cuobjdump = shutil.which("cuobjdump") or shutil.which("cuobjdump", path=cuda_bin)
+    if not nvcc or not cuobjdump:
+        pytest.skip("nvcc / cuobjdump not found")
+    src = tmp_path / "probe.cu"
+    src.write_text('#include "hp_sweep_common.cuh"\n'
+                   "__global__ void probe(unsigned int* flag) { hp_raise_abort(flag); }\n")
+    cubin = tmp_path / "probe.cubin"
+    subprocess.check_call([nvcc, "-gencode", "arch=compute_100a,code=sm_100a", "-cubin",
+                           "-I", os.path.join(ROOT, "helmholtz_preconditioner_b200", "csrc"), "-o", str(cubin), str(src)])
+    sass = subprocess.check_output([cuobjdump, "-sass", str(cubin)], text=True)
+    instr = [ln.split("*/", 1)[1].split(";")[0].strip() for ln in sass.splitlines() if re.match(r"\s*/\*[0-9a-f]{4}\*/", ln)]
+    assert not [i for i in instr if re.match(r"CALL\b", i)], sass
+    assert len([i for i in instr if re.match(r"ATOMG\S*\.EXCH\b", i)]) == 2, sass

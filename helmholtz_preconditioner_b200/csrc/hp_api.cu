@@ -114,8 +114,10 @@ extern "C" int hp_context_clone(hp_solver* s, hp_solver** out, void* stream) {
     *out = nullptr;
     if (!s->f_low || !s->bar) { hp_set_error("hp_context_clone: preconditioner not set up"); return 1; }
     cudaStream_t st = (cudaStream_t)stream;
+    hp_solver* owner = s->is_view ? s->parent : s;
     hp_solver* c = new hp_solver(*s);
     c->is_view = 1;
+    c->parent = nullptr; c->live_ctx = 0;                  // counted in the owner once the scratch exists
     // Sweeps of a context are plain cluster launches.  A cooperative launch is ordered against all other work of the process
     // on the device (measured: with the sweep of one group queued behind a stream-level wait for another GPU, the cooperative
     // launch of the next group blocks its host thread inside the launch call, and two processes then wait for each other).
@@ -133,13 +135,24 @@ extern "C" int hp_context_clone(hp_solver* s, hp_solver** out, void* stream) {
         hp_set_error("hp_context_clone: allocation of the sweep scratch failed: %s", cudaGetErrorString(cudaGetLastError()));
         return fail();
     }
+    c->parent = owner;
+    owner->live_ctx++;
     *out = c;
     return 0;
+}
+
+// A context keeps the addresses of its owner's factorisation: refactoring the owner while one is open would leave the
+// context pointing at freed memory, so the calls that replace the factorisation refuse until every context is destroyed.
+static int hp_refuse_with_contexts(const hp_solver* s, const char* what) {
+    if (s->live_ctx <= 0) return 0;
+    hp_set_error("%s: %d context(s) made by hp_context_clone still use this factorisation; destroy them first", what, s->live_ctx);
+    return 1;
 }
 
 extern "C" int hp_destroy(hp_solver* s) {
     if (!s) return 0;
     if (s->is_view) {
+        if (s->parent) s->parent->live_ctx--;
         cudaFree(s->xch); cudaFree(s->bar); cudaFree(s->TF); cudaFree(s->TFm); cudaFree(s->fc_work); cudaFree(s->dbg);
         for (cudaEvent_t e : s->prof_ev) cudaEventDestroy(e);
         delete s;
@@ -158,6 +171,7 @@ extern "C" int hp_destroy(hp_solver* s) {
 extern "C" int hp_precond_setup(hp_solver* s, int P, int K, int m_lo, int m_hi, void* stream) {
     if (!s) { hp_set_error("hp_precond_setup: null solver"); return 1; }
     if (s->is_view) { hp_set_error("hp_precond_setup: a context made by hp_context_clone shares the factorisation of its parent"); return 1; }
+    if (hp_refuse_with_contexts(s, "hp_precond_setup")) return 1;
     if (m_lo == 0 && m_hi == 0) { m_lo = s->b + 1; m_hi = s->n; }
     if (m_lo < s->b + 1 || m_hi > s->n) {
         hp_set_error("hp_precond_setup: strips must lie in %d..%d, got %d..%d", s->b + 1, s->n, m_lo, m_hi);
@@ -193,12 +207,15 @@ extern "C" int hp_debug_phases(hp_solver* s, int on, long long* out_host) {
 // front block used by the next hp_precond_setup: 0 = block diagonal (the reference's get_A_FF_block), 1 = coupled
 extern "C" int hp_set_front_mode(hp_solver* s, int mode) {
     if (!s || mode < 0 || mode > 1) { hp_set_error("hp_set_front_mode: mode must be 0 or 1"); return 1; }
+    // the front solves read front_mode at once: switching it under a factorisation of the other mode is a refactoring
+    if (mode != s->front_mode && hp_refuse_with_contexts(s, "hp_set_front_mode")) return 1;
     s->front_mode = mode;
     return 0;
 }
 // re-factor the front block alone with another mode; the strip factorisation is kept
 extern "C" int hp_precond_set_front(hp_solver* s, int mode, void* stream) {
     if (s && s->is_view) { hp_set_error("hp_precond_set_front: not on a context made by hp_context_clone"); return 1; }
+    if (s && hp_refuse_with_contexts(s, "hp_precond_set_front")) return 1;
     if (hp_set_front_mode(s, mode)) return 1;
     cudaStream_t st = (cudaStream_t)stream;
     HP_CUDA(cudaMemsetAsync(s->status, 0, sizeof(int), st));

@@ -80,6 +80,8 @@ struct hp_solver {
     size_t xch_count = 0, bar_count = 0;   // complex numbers of xch, words of bar (hp_context_clone allocates the same)
     int coop = 1;                 // 1: sweeps are cooperative launches (the driver checks co-residency); contexts: 0, see hp_context_clone
     int is_view = 0;              // 1: created by hp_context_clone, owns only its sweep scratch (xch, bar, TF, TFm, fc_work)
+    hp_solver* parent = nullptr;  // context: the solver whose factorisation it shares
+    int live_ctx = 0;             // solver: contexts cloned from it and not destroyed yet (they hold its pointers)
     long long* dbg = nullptr;     // optional per-phase cycle counters of the sweep kernel [G][8]
     int sweep_variant = 0;        // 0 = automatic; classic layout: 1 direct, 2 TMA staged, 3 pipelined; cluster layout: 4
     int layout_mode = 0;          // 0 = automatic (cluster layout when a partition exists), 1 = classic, 2 = cluster

@@ -82,6 +82,11 @@ class SlabSolver:
         for q in dist.batch_isend_irecv(ops):
             q.wait()
 
+    def _post(self, ops):
+        """batched non-blocking sends that the caller waits for later; returns their work handles"""
+        CommStats.calls += 1
+        return dist.batch_isend_irecv(ops)
+
     def _row(self, j, buf=None):
         """view of global row j inside the ghosted buffer (j0-1 <= j <= j1)."""
         o = (j - (self.j0 - 1)) * self.n
@@ -212,8 +217,7 @@ class SlabSolver:
                     for bf in bufs:
                         self.s.sweep_forward_buf(bf, row0, self.m_lo, m_to)
             if r < w - 1:
-                CommStats.calls += 1
-                sends += dist.batch_isend_irecv([dist.P2POp(dist.isend, self._row(self.j1, bf), r + 1, self.group) for bf in bufs])
+                sends += self._post([dist.P2POp(dist.isend, self._row(self.j1, bf), r + 1, self.group) for bf in bufs])
         for q in sends:                                      # the rows come back in the backward chain
             q.wait()
         sends = []
@@ -228,8 +232,7 @@ class SlabSolver:
                     for bf in bufs:
                         self.s.sweep_backward_buf(bf, row0, self.m_hi, self.m_lo, diag)
             if r > 0:
-                CommStats.calls += 1
-                sends += dist.batch_isend_irecv([dist.P2POp(dist.isend, self._row(self.j0, bf), r - 1, self.group) for bf in bufs])
+                sends += self._post([dist.P2POp(dist.isend, self._row(self.j0, bf), r - 1, self.group) for bf in bufs])
             else:
                 for i in grp:
                     if R > 1:

@@ -44,7 +44,9 @@ int hp_destroy(hp_solver* s);
  * private copy of the sweep scratch (exchange ring, abort flags, parked front solutions T_F u_F of code.py:364), so that
  * applications of algo2_4 (code.py:356-385) issued through different contexts can be in flight on different streams at
  * once.  The reference has no counterpart (one Python thread); slab.py uses one context per group of right-hand sides.
- * `s` must outlive the context; hp_destroy(context) frees the scratch only; setup calls on a context are refused. */
+ * `s` must outlive the context; hp_destroy(context) frees the scratch only; setup calls on a context are refused.
+ * While a context of `s` is open, hp_precond_setup, hp_precond_set_front and a change of hp_set_front_mode on `s` are
+ * refused too (they would replace the factorisation the context points to). */
 int hp_context_clone(hp_solver* s, hp_solver** out, void* stream);
 
 /* ---- operator A ---------------------------------------------------------------------------------- */

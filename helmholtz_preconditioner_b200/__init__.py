@@ -8,7 +8,7 @@ from .fields import (init_c1_f1, init_c1_f2, init_c1_mat, init_c2_f1, init_c2_f2
 
 def __getattr__(name):
     # solver.py needs torch; keep `import helmholtz_preconditioner_b200` light for the host-only tests
-    if name in ("HelmholtzSolver", "DeviceCSR", "SolveResult", "run_solver", "build_A_matrix", "algo2_3", "algo2_4", "get_Hm", "get_A_FF_block"):
+    if name in ("HelmholtzSolver", "DeviceCSR", "SolveResult", "run_solver", "run_solver_many", "build_A_matrix", "algo2_3", "algo2_4", "get_Hm", "get_A_FF_block"):
         from . import solver
         return getattr(solver, name)
     if name in ("gmres", "gmres_batch", "DeviceVectors", "lartg"):

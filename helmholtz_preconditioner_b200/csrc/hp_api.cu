@@ -266,7 +266,7 @@ extern "C" int hp_precond_apply(hp_solver* s, const double* f_dev, double* u_dev
 }
 
 // algo2_4 for R right-hand sides with ONE pass over the strip generators per sweep direction (csrc/hp_sweep4m.cu).
-// R must be 1, 2, 4 or 8 and at most hp_multi_max(s).
+// R must be 1, 2, 4 or 8 and at most hp_multi_max(s).  Slots whose two pointers are NULL are skipped (masked).
 extern "C" int hp_precond_apply_multi(hp_solver* s, int R, const double* const* f_devs, double* const* u_devs, int diag_mode,
                                       void* stream) {
     if (!s || !f_devs || !u_devs) { hp_set_error("hp_precond_apply_multi: null argument"); return 1; }
@@ -279,12 +279,24 @@ extern "C" int hp_precond_apply_multi(hp_solver* s, int R, const double* const* 
         hp_set_error("hp_precond_apply_multi: R must be a power of two <= %d, got %d", hp_multi_max(s), R);
         return 1;
     }
+    // a slot with f_devs[r] == u_devs[r] == NULL is inactive: the launch carries the other slots at their own indices
+    int active = 0;
+    for (int r = 0; r < R; ++r) {
+        if (!f_devs[r] != !u_devs[r]) {
+            hp_set_error("hp_precond_apply_multi: slot %d has %s input but %s output (both or neither must be NULL)", r,
+                         f_devs[r] ? "an" : "no", u_devs[r] ? "an" : "no");
+            return 1;
+        }
+        active += u_devs[r] != nullptr;
+    }
+    if (!active) { hp_set_error("hp_precond_apply_multi: all %d slots are empty", R); return 1; }
     cudaStream_t st = (cudaStream_t)stream;
     const int n = s->n, b = s->b;
     const size_t tf = (size_t)b * n;
     if (!s->TFm) HP_CUDA(cudaMalloc(&s->TFm, sizeof(cplx) * tf * 8));
     int rc;
     for (int r = 0; r < R; ++r) {
+        if (!u_devs[r]) continue;
         if (f_devs[r] != u_devs[r])
             HP_CUDA(cudaMemcpyAsync(u_devs[r], f_devs[r], sizeof(cplx) * (size_t)n * n, cudaMemcpyDeviceToDevice, st));
         if ((rc = hp_front_begin(s, u_devs[r], stream))) return rc;
@@ -295,6 +307,7 @@ extern "C" int hp_precond_apply_multi(hp_solver* s, int R, const double* const* 
         if ((rc = hp_sweep_backward_multi(s, R, u_devs, n, b + 1, diag_mode, stream))) return rc;
     }
     for (int r = 0; r < R; ++r) {
+        if (!u_devs[r]) continue;
         HP_CUDA(cudaMemcpyAsync(s->TF, s->TFm + r * tf, sizeof(cplx) * tf, cudaMemcpyDeviceToDevice, st));
         if ((rc = hp_front_end(s, u_devs[r], stream))) return rc;
     }

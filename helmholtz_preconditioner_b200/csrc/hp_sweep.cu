@@ -440,6 +440,9 @@ int hp_sweep_launch_multi(hp_solver* s, int mode, int R, cplx* const* um, int m_
     const int kernel = hp_multi_kernel(s, R);
     if (!kernel) { hp_set_error("sweep: %d right-hand sides per launch not supported by this layout", R); return 1; }
     const bool tensor = kernel == 2;
+    int first = 0;                                       // null entries are inactive slots (hp_sweep4_dev.cuh: ldcg_slot)
+    while (first < R && !um[first]) ++first;
+    if (first == R) { hp_set_error("sweep: all %d right-hand-side slots of the launch are empty", R); return 1; }
     int lo = mode == 1 ? m_to : m_from, hi = mode == 1 ? m_from : m_to;
     if (lo > hi) return 0;
     if (lo < s->m_lo || hi > s->m_hi) {
@@ -452,7 +455,7 @@ int hp_sweep_launch_multi(hp_solver* s, int mode, int R, cplx* const* um, int m_
     a.leaf_start = s->leaf_start; a.leaf_q = s->leaf_q; a.sep = s->sep;
     a.packets = s->packets; a.mleaf = s->mleaf; a.rsep = s->rsep; a.m_lo = s->m_lo;
     a.mode = mode; a.m_from = m_from; a.m_to = m_to; a.diag_mode = diag_mode;
-    a.u = um[0]; a.vin = nullptr; a.yout = nullptr;
+    a.u = um[first]; a.vin = nullptr; a.yout = nullptr;     // not read by hp_sweep4d / hp_sweep4m
     for (int r = 0; r < HP_RMAX; ++r) a.um[r] = r < R ? um[r] : nullptr;
     a.xch = s->xch; a.bar = s->bar;
     a.oGP = 0; a.oXS = (size_t)L.G * s->b * R; a.oGR = a.oVS = 0;

@@ -65,6 +65,13 @@ __device__ __forceinline__ void mbar_wait_acq4(unsigned long long* bar, unsigned
 __device__ __forceinline__ void mbar_arrive_local(unsigned long long* bar) {
     asm volatile("mbarrier.arrive.relaxed.cta.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
+// field accesses of the multi-vector kernels: a right-hand-side slot whose field pointer is null is inactive (masked),
+// every load of it reads 0 and every store is dropped.  A per-lane predicate, nothing else: the zero column runs through
+// the products like any other input, so active slots compute exactly what they compute in a full launch.
+__device__ __forceinline__ cplx ldcg_slot(const cplx* u, size_t i) { return u ? ldcg(u + i) : cmake(0.0, 0.0); }
+__device__ __forceinline__ void st_slot(cplx* u, size_t i, cplx v) {
+    if (u) u[i] = v;
+}
 __device__ __forceinline__ void ring_fill4(unsigned char* dst, const cplx* src, unsigned int bytes, unsigned long long* bar) {
     mbar_expect_tx(bar, bytes);
     for (unsigned int o = 0; o < bytes; o += HP_BULK_CHUNK)

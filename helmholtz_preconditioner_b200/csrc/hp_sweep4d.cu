@@ -173,19 +173,19 @@ __global__ void __launch_bounds__(HP4D_THREADS, 1) hp_sweep4d_kernel(HpSweepArgs
 #pragma unroll
             for (int i = 0; i < 2; ++i) {
                 cplx* u = i ? u1 : u0;
-                if (a_mode == 0) vsb[i] = ldcg(u + (size_t)(m0 - 1) * n + sep_col);
+                if (a_mode == 0) vsb[i] = ldcg_slot(u, (size_t)(m0 - 1) * n + sep_col);
                 else {
-                    usbase[i] = ldcg(u + (size_t)(m0 - 1) * n + sep_col);
+                    usbase[i] = ldcg_slot(u, (size_t)(m0 - 1) * n + sep_col);
                     vsb[i] = usbase[i];
-                    if (m0 < n) vsb[i] = cfma(cscale(sg, cmul(hp_rowfac(a, m0), cis1s)), ldcg(u + (size_t)m0 * n + sep_col), vsb[i]);
+                    if (m0 < n) vsb[i] = cfma(cscale(sg, cmul(hp_rowfac(a, m0), cis1s)), ldcg_slot(u, (size_t)m0 * n + sep_col), vsb[i]);
                 }
             }
         }
         auto sep_output = [&](int m_prev, int i, cplx ys) {   // y_s = x_l[b-1] of strip m_prev, right-hand side 2 ft + i
             if (k != 0) return;
             cplx* u = i ? u1 : u0;
-            if (a_mode == 0) u[(size_t)m_prev * n + sep_col] = cfms(o_c, ys, o_usep[i]);
-            else u[(size_t)(m_prev - 1) * n + sep_col] = a_diag == 0 ? csub(o_usbase[i], ys) : ys;
+            if (a_mode == 0) st_slot(u, (size_t)m_prev * n + sep_col, cfms(o_c, ys, o_usep[i]));
+            else st_slot(u, (size_t)(m_prev - 1) * n + sep_col, a_diag == 0 ? csub(o_usbase[i], ys) : ys);
         };
         const int nks_b = (b3 + 3) >> 2, ks_per = (nks_b + HP4_CW - 1) / HP4_CW;       // k-steps of P = R X3, split over the warps
         const int ntile_e = (b + 7) >> 3;                                              // entry tiles (2 for b = 12)
@@ -205,8 +205,8 @@ __global__ void __launch_bounds__(HP4D_THREADS, 1) hp_sweep4d_kernel(HpSweepArgs
 #pragma unroll
                 for (int i = 0; i < 2; ++i) {
                     cplx* u = i ? u1 : u0;
-                    if (a_mode == 0) usep[i] = ldcg(u + (size_t)m * n + sep_col);
-                    else if (more) usep[i] = ldcg(u + (size_t)(mn - 1) * n + sep_col);
+                    if (a_mode == 0) usep[i] = ldcg_slot(u, (size_t)m * n + sep_col);
+                    else if (more) usep[i] = ldcg_slot(u, (size_t)(mn - 1) * n + sep_col);
                 }
             }
             // ---- x-independent part: the K partial sums of gl (DSMEM) and gf (L2, poll warp), split over the warps
@@ -456,11 +456,11 @@ __global__ void __launch_bounds__(HP4D_THREADS, 1) hp_sweep4d_kernel(HpSweepArgs
 #pragma unroll
             for (int i = 0; i < 2; ++i) {
                 cplx* u = i ? u1 : u0;
-                if (a_mode == 0) vbr[i] = ldcg(u + (size_t)(m0 - 1) * n + c);
+                if (a_mode == 0) vbr[i] = ldcg_slot(u, (size_t)(m0 - 1) * n + c);
                 else {
-                    ubase[i] = ldcg(u + (size_t)(m0 - 1) * n + c);
+                    ubase[i] = ldcg_slot(u, (size_t)(m0 - 1) * n + c);
                     vbr[i] = ubase[i];
-                    if (m0 < n) vbr[i] = cfma(cscale(sg, cmul(hp_rowfac(a, m0), cis1)), ldcg(u + (size_t)m0 * n + c), vbr[i]);
+                    if (m0 < n) vbr[i] = cfma(cscale(sg, cmul(hp_rowfac(a, m0), cis1)), ldcg_slot(u, (size_t)m0 * n + c), vbr[i]);
                 }
                 vb[(size_t)(2 * ft + i) * CWV + oc] = vbr[i];
             }
@@ -489,8 +489,8 @@ __global__ void __launch_bounds__(HP4D_THREADS, 1) hp_sweep4d_kernel(HpSweepArgs
 #pragma unroll
                 for (int i = 0; i < 2; ++i) {
                     cplx* u = i ? u1 : u0;
-                    if (a_mode == 0) unx[i] = ldcg(u + (size_t)m * n + c);
-                    else if (more) unx[i] = ldcg(u + (size_t)(mn - 1) * n + c);
+                    if (a_mode == 0) unx[i] = ldcg_slot(u, (size_t)m * n + c);
+                    else if (more) unx[i] = ldcg_slot(u, (size_t)(mn - 1) * n + c);
                 }
             }
             if (DBG && (ot == 0 || ot == 128)) tprev = clock64();
@@ -605,8 +605,8 @@ __global__ void __launch_bounds__(HP4D_THREADS, 1) hp_sweep4d_kernel(HpSweepArgs
                         for (int i = 0; i < 2; ++i) {
                             cplx* u = i ? u1 : u0;
                             v[i] = cfma(coefc, corr[i], vbr[i]);
-                            if (a_mode == 0) u[(size_t)mp * n + c] = v[i];
-                            else u[(size_t)(mp - 1) * n + c] = a_diag == 0 ? cadd(csub(ubase_prev[i], y0prev[i]), corr[i]) : csub(y0prev[i], corr[i]);
+                            if (a_mode == 0) st_slot(u, (size_t)mp * n + c, v[i]);
+                            else st_slot(u, (size_t)(mp - 1) * n + c, a_diag == 0 ? cadd(csub(ubase_prev[i], y0prev[i]), corr[i]) : csub(y0prev[i], corr[i]));
                         }
                     }
                 }

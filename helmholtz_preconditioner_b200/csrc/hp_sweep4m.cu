@@ -139,12 +139,13 @@ __global__ void __launch_bounds__(HP4_THREADS, 1) hp_sweep4m_kernel(HpSweepArgs 
         constexpr int NPASS = (HP_BMAX + EPP - 1) / EPP;
         cplx* const u = a.um[rr];
         const bool is_sep = has_sep && ks == 0 && e_lo == (b - 1) % EPP;
+        const bool sep_io = is_sep && u != nullptr;          // field accesses of an empty slot are skipped (reads give 0)
         const int sep_pass = (b - 1) / EPP;
         const int sep_col = has_sep ? a.sep[l] : 0;
         const cplx cis1s = is_sep ? a.is1t[2 * (sep_col + 1)] : cmake(0.0, 0.0);
         cplx usbase = cmake(0.0, 0.0), vsb = cmake(0.0, 0.0);
         cplx o_usep = cmake(0.0, 0.0), o_c = cmake(0.0, 0.0), o_usbase = cmake(0.0, 0.0);
-        if (is_sep) {
+        if (sep_io) {
             if (a_mode == 0) vsb = ldcg(u + (size_t)(m0 - 1) * n + sep_col);
             else {
                 usbase = ldcg(u + (size_t)(m0 - 1) * n + sep_col);
@@ -153,7 +154,7 @@ __global__ void __launch_bounds__(HP4_THREADS, 1) hp_sweep4m_kernel(HpSweepArgs 
             }
         }
         auto sep_output = [&](int m_prev, cplx ys) {          // y_s = x_l[b-1] of strip m_prev
-            if (k != 0) return;
+            if (k != 0 || !sep_io) return;
             if (a_mode == 0) u[(size_t)m_prev * n + sep_col] = cfms(o_c, ys, o_usep);
             else u[(size_t)(m_prev - 1) * n + sep_col] = a_diag == 0 ? csub(o_usbase, ys) : ys;
         };
@@ -169,8 +170,8 @@ __global__ void __launch_bounds__(HP4_THREADS, 1) hp_sweep4m_kernel(HpSweepArgs 
             cplx usep = cmake(0.0, 0.0), cs = cmake(0.0, 0.0);
             if (is_sep) {
                 cs = cmul(hp_rowfac(a, a_mode == 1 ? mn : m), cis1s);
-                if (a_mode == 0) usep = ldcg(u + (size_t)m * n + sep_col);
-                else if (more) usep = ldcg(u + (size_t)(mn - 1) * n + sep_col);
+                if (a_mode == 0) { if (sep_io) usep = ldcg(u + (size_t)m * n + sep_col); }
+                else if (more && sep_io) usep = ldcg(u + (size_t)(mn - 1) * n + sep_col);
             }
             // ---- x-independent part of rho_l(it): own-cluster gl partials (DSMEM) + gf partials of leaf l+1 (L2)
             cplx pre[NPASS];
@@ -412,13 +413,15 @@ __global__ void __launch_bounds__(HP4_THREADS, 1) hp_sweep4m_kernel(HpSweepArgs 
         const int cpart = ot & 7, oc = ot >> 3;
         const int rr = cpart % RT, ks = cpart / RT;
         const bool col = oc < ncols, colw = col && ks == 0;
+        const bool col_io = col && a.um[rr] != nullptr;      // field accesses of an empty slot are skipped (reads give 0)
         const int c = c0 + oc;
         cplx* const u = a.um[rr];
         const cplx cis1 = col ? a.is1t[2 * (c + 1)] : cmake(0.0, 0.0);
         cplx vbr = cmake(0.0, 0.0), y0prev = cmake(0.0, 0.0), coefc = cmake(0.0, 0.0), ubase = cmake(0.0, 0.0),
              ubase_prev = cmake(0.0, 0.0);
         if (col) {
-            if (a_mode == 0) vbr = ldcg(u + (size_t)(m0 - 1) * n + c);
+            if (!col_io) {
+            } else if (a_mode == 0) vbr = ldcg(u + (size_t)(m0 - 1) * n + c);
             else {
                 ubase = ldcg(u + (size_t)(m0 - 1) * n + c);
                 vbr = ubase;
@@ -442,7 +445,7 @@ __global__ void __launch_bounds__(HP4_THREADS, 1) hp_sweep4m_kernel(HpSweepArgs 
             const cplx* Gprev = reinterpret_cast<const cplx*>(ringG + (size_t)((it + 2) % 3) * pl.g_st);
             const cplx rf_it = hp_rowfac(a, a_mode == 1 ? mn : m);
             cplx unx = cmake(0.0, 0.0);
-            if (col && live) {
+            if (col_io && live) {
                 if (a_mode == 0) unx = ldcg(u + (size_t)m * n + c);
                 else if (more) unx = ldcg(u + (size_t)(mn - 1) * n + c);
             }
@@ -509,7 +512,7 @@ __global__ void __launch_bounds__(HP4_THREADS, 1) hp_sweep4m_kernel(HpSweepArgs 
                 if (col && live)
                     for (int d = ks; d < K; d += KS)
                         st_async_cplx(mapa_u32(smem_u32(v_leaf + ((size_t)par * RT + rr) * QP + lc0 + oc), d), v, mapa_u32(smem_u32(&barV[par]), d));
-                if (colw) {
+                if (colw && col_io) {
                     if (a_mode == 0) u[(size_t)mp * n + c] = v;
                     else {
                         cplx un = a_diag == 0 ? cadd(csub(ubase_prev, y0prev), corr) : csub(y0prev, corr);

@@ -229,12 +229,14 @@ def gmres(matvec, psolve, b, *, vec, rtol=1e-5, atol=0.0, restart=20, maxiter=No
         return done.value
 
 
-def gmres_batch(matvec, psolve_batch, bs, *, vec, matvec_batch=None, **kw):
+def gmres_batch(matvec, psolve_batch, bs, *, vec, matvec_batch=None, with_index=False, **kw):
     """The same iteration for several right-hand sides advanced in lock step.  Every round collects the pending request of
     each unfinished system and serves them together: preconditioner requests go to psolve_batch as a list (one
     multi-right-hand-side sweep on one GPU; pipelined through the slabs in slab.py), operator requests to matvec_batch
     (halo rows of all systems in one exchange), norms and Gram-Schmidt steps to the batched reductions of DeviceVectors
-    (one all-reduce per Arnoldi column for all systems).  Returns [(x, info, hist), ...] in the order of `bs`."""
+    (one all-reduce per Arnoldi column for all systems).  Returns [(x, info, hist), ...] in the order of `bs`.
+    with_index=True: psolve_batch receives (i, x, out) triples, i the index of the system in `bs` (a caller can then
+    keep every system in its own slot of the sweep launch); default: (x, out) pairs."""
     gens = [gmres_steps(b, vec=vec, **kw) for b in bs]
     results = [None] * len(bs)
     reqs = {}
@@ -260,7 +262,7 @@ def gmres_batch(matvec, psolve_batch, bs, *, vec, matvec_batch=None, **kw):
             import threading
             print(f"[gmres_batch {threading.current_thread().name}] {key} x{len(idx)}", file=sys.stderr, flush=True)
         if kind == "M":
-            psolve_batch([(reqs[i][1], reqs[i][2]) for i in idx])
+            psolve_batch([(i, reqs[i][1], reqs[i][2]) if with_index else (reqs[i][1], reqs[i][2]) for i in idx])
             vals = [None] * len(idx)
         elif kind == "A":
             if matvec_batch is not None:

@@ -18,11 +18,12 @@ import numpy as np
 import torch
 
 from . import _lib, fields
-from .gmres import DeviceVectors, gmres
+from .gmres import DeviceVectors, gmres, gmres_batch
 
 DIAG_MODES = {"reference": 0, "paper": 1}
 LAYOUT_MODES = {"auto": 0, "classic": 1, "cluster": 2}
 FRONT_MODES = {"blockdiag": 0, "coupled": 1}
+HP_RMAX = 8                       # right-hand sides of the widest sweep launch (csrc/hp_sweep_common.cuh)
 
 
 def _ptr(t):
@@ -258,18 +259,48 @@ class HelmholtzSolver:
 
     @staticmethod
     def _ptr_array(ts):
-        return (C.c_void_p * len(ts))(*[t.data_ptr() for t in ts])
+        return (C.c_void_p * len(ts))(*[0 if t is None else t.data_ptr() for t in ts])
 
     def precond_apply_multi(self, fs, outs, diag="reference"):
-        """algo2_4 on R = len(fs) vectors with one pass over the strip generators per sweep (R in {1, 2, 4, 8})."""
+        """algo2_4 on R = len(fs) vectors with one pass over the strip generators per sweep (R in {1, 2, 4, 8}).
+        fs[i] = outs[i] = None leaves slot i of the launch empty (masked)."""
         self._on_device()
         _lib.check(self.lib.hp_precond_apply_multi(self.handle, len(fs), self._ptr_array(fs), self._ptr_array(outs), DIAG_MODES[diag],
                                                    _stream()), "hp_precond_apply_multi")
         return outs
 
-    def precond_apply_batch(self, pairs, diag="reference"):
-        """out_i = M x_i for every (x_i, out_i) of `pairs`, in groups of batch_group() right-hand sides per launch"""
+    def precond_apply_slots(self, slots, diag="reference"):
+        """out = M x for every entry (x, out) of `slots` in ONE launch per sweep direction, entry i in slot i of the
+        launch; None entries are empty slots.  len(slots) is the launch width (1, or a power of two the layout can carry,
+        multi_kernel(len(slots)) != 0).  An active slot's result does not depend on what the other slots hold."""
+        if len(slots) == 1:
+            if slots[0] is None:
+                raise _lib.HelmholtzB200Error("precond_apply_slots: the only slot of the launch is empty")
+            self.precond_apply(slots[0][0], out=slots[0][1], diag=diag)
+            return
+        self.precond_apply_multi([None if p is None else p[0] for p in slots], [None if p is None else p[1] for p in slots],
+                                 diag=diag)
+
+    def _widest(self):
+        """right-hand sides of the widest launch in use (multi_max, capped by max_group)"""
+        return self.batch_group(HP_RMAX)
+
+    def precond_apply_batch(self, pairs, diag="reference", pad=False):
+        """out_i = M x_i for every (x_i, out_i) of `pairs`.  pad=False: in groups of batch_group() right-hand sides per
+        launch (7 pairs: launches of 4 + 2 + 1).  pad=True: the widest launch takes min(remaining, widest) pairs and is
+        padded with empty slots up to the smallest width that holds them and that the layout supports (7 pairs: one
+        8-wide launch with one empty slot; 3 pairs: one 4-wide launch)."""
         i = 0
+        if pad:
+            cap = self._widest()
+            while i < len(pairs):
+                take = min(len(pairs) - i, cap)
+                w = 1
+                while w < take or (w > 1 and w < cap and not self.multi_kernel(w)):
+                    w *= 2
+                self.precond_apply_slots(list(pairs[i:i + take]) + [None] * (w - take), diag=diag)
+                i += take
+            return
         while i < len(pairs):
             g = self.batch_group(len(pairs) - i)
             if g == 1:
@@ -279,11 +310,12 @@ class HelmholtzSolver:
             i += g
 
     def sweep_forward_multi_buf(self, bufs, row0, m_from, m_to):
-        arr = (C.c_void_p * len(bufs))(*[self._base(t, row0) for t in bufs])
+        """one multi-vector forward sweep over strips m_from..m_to; a None entry is an empty slot"""
+        arr = (C.c_void_p * len(bufs))(*[0 if t is None else self._base(t, row0) for t in bufs])
         _lib.check(self.lib.hp_sweep_forward_multi(self.handle, len(bufs), arr, m_from, m_to, _stream()), "hp_sweep_forward_multi")
 
     def sweep_backward_multi_buf(self, bufs, row0, m_from, m_to, diag="reference"):
-        arr = (C.c_void_p * len(bufs))(*[self._base(t, row0) for t in bufs])
+        arr = (C.c_void_p * len(bufs))(*[0 if t is None else self._base(t, row0) for t in bufs])
         _lib.check(self.lib.hp_sweep_backward_multi(self.handle, len(bufs), arr, m_from, m_to, DIAG_MODES[diag], _stream()),
                    "hp_sweep_backward_multi")
 
@@ -465,3 +497,76 @@ def run_solver(n, b, wave_num, const, alpha, init_func=fields.init_c1_f1, plot_s
         print("Initialization time = " + str(t1 - t0))
         print("GMRES solve time = " + str(t2 - t1))
     return SolveResult(u, hist, len(hist), info, t1 - t0, t2 - t1, s)
+
+
+def _source_fields(f_mats, n, device):
+    """(S, n, n) / (S, n*n) array or tensor, or a list of (n, n) / (n*n,) fields -> list of (n*n,) device tensors"""
+    items = list(f_mats) if isinstance(f_mats, (list, tuple)) else [f_mats[i] for i in range(f_mats.shape[0])]
+    fs = [_as_device_field(f, device) for f in items]
+    for i, f in enumerate(fs):
+        if f.numel() != n * n:
+            raise ValueError(f"source {i} has {f.numel()} entries, expected n*n = {n * n}")
+    return fs
+
+
+def run_solver_many(n, b, wave_num, const, alpha, f_mats, init_func=fields.init_c1_f1, *, c_mat=None, diag="reference",
+                    precond_input="rhs", front="blockdiag", rtol=1e-3, restart=20, maxiter=None, device=None, P=0, K=0,
+                    verbose=True, solver=None):
+    """run_solver for several sources (right-hand sides) of one medium: the solver is set up once, and the sources are
+    solved in waves of as many as one sweep launch carries (multi_max; 1 = one source at a time).
+
+    f_mats: (S, n, n) or (S, n*n) array or tensor, or a list of such fields.  c_mat defaults to init_func's.  The other
+    arguments mean what they mean for run_solver.  Within a wave, source i always occupies slot i of the sweep launch;
+    the slots of sources that have converged, or that do not ask for M x in a round, are left empty.  So every
+    preconditioner round is one launch per sweep direction, and a source's result does not depend on which sources
+    share its wave (bit for bit, given its slot).
+
+    Returns one SolveResult per source in input order: init_time is the shared set-up time, solve_time the wall time of
+    the source's wave; u, residuals, niter and info are the source's own."""
+    _lib.require_device()
+    t0 = time.time()
+    omega = 2 * np.pi * wave_num + 1j * alpha
+    if c_mat is None and solver is None:
+        c_mat = init_func(omega, n)[0]
+    s = solver if solver is not None else HelmholtzSolver(n, b, omega, const, c_mat, device=device)
+    fs = _source_fields(f_mats, n, s.device)
+    if solver is None:
+        s.setup_preconditioner(P, K, front=front)
+    if precond_input not in ("rhs", "vector"):
+        raise ValueError("precond_input must be 'rhs' or 'vector'")
+    torch.cuda.synchronize(s.device)
+    t1 = time.time()
+    W = s._widest()
+    vec = DeviceVectors(n * n, s.device, restart=restart)
+    results = []
+    for w0 in range(0, len(fs), W):
+        tw = time.time()
+        wave = fs[w0:w0 + W]
+        Mf = None
+        if precond_input == "rhs":
+            # as in run_solver, M f is computed once and copied: one launch for the whole wave
+            Mf = [torch.empty_like(f) for f in wave]
+            s.precond_apply_slots([(f, m) for f, m in zip(wave, Mf)] + [None] * (W - len(wave)), diag=diag)
+
+        def psolve_batch(reqs, Mf=Mf):
+            if Mf is not None:
+                for i, _, out in reqs:
+                    vec.scale_copy(1.0, Mf[i], out)
+                return
+            slots = [None] * W
+            for i, x, out in reqs:
+                slots[i] = (x, out)
+            s.precond_apply_slots(slots, diag=diag)
+
+        outs = gmres_batch(lambda x, out: s.matvec(x, out), psolve_batch, wave, vec=vec, with_index=True, rtol=rtol,
+                           restart=restart, maxiter=maxiter, health=s.check_status)
+        s.check_status()
+        t_wave = time.time() - tw
+        for j, (u, info, hist) in enumerate(outs):
+            results.append(SolveResult(u, hist, len(hist), info, t1 - t0, t_wave, s))
+            if verbose:
+                print(f"source {w0 + j}: GMRES iterations with preconditioner: {len(hist)} (info {info})")
+    if verbose:
+        print("Initialization time = " + str(t1 - t0))
+        print("GMRES solve time = " + str(time.time() - t1))
+    return results

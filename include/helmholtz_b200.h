@@ -124,8 +124,14 @@ int hp_multi_max(hp_solver* s);
 /* Kernel that one launch carrying R right-hand sides runs (the choice hp_sweep_forward_multi / hp_sweep_backward_multi
  * make): 2 = hp_sweep4d (FP64 tensor cores, R = 8), 1 = hp_sweep4m, 0 = none (R is not supported by this layout). */
 int hp_multi_kernel(hp_solver* s, int R);
+/* Masked slots: an entry u_devs[r] == NULL is an inactive slot of the launch.  Its loads read 0 and nothing is stored
+ * for it; the other slots keep their index r and their results are bit for bit those of a launch of the same width in
+ * which every slot is active, whatever the other slots hold.  R keeps the rules above; at least one entry must be
+ * non-NULL, otherwise the call fails. */
 int hp_sweep_forward_multi(hp_solver* s, int R, double* const* u_devs, int m_from, int m_to, void* stream);
 int hp_sweep_backward_multi(hp_solver* s, int R, double* const* u_devs, int m_from, int m_to, int diag_mode, void* stream);
+/* f_devs[r] and u_devs[r] are both NULL (inactive slot: no copy, no front solve) or both non-NULL; at least one slot must
+ * be active.  Any other combination fails without launching anything. */
 int hp_precond_apply_multi(hp_solver* s, int R, const double* const* f_devs, double* const* u_devs, int diag_mode, void* stream);
 /* y = T_m v : last n entries of H_m^{-1} [0; v]  (lu_Hm_ra[m-b-1].solve(u_temp)[-n:], code.py:370) */
 int hp_strip_apply(hp_solver* s, int m, const double* v_dev, double* y_dev, void* stream);

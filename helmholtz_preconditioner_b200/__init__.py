@@ -2,7 +2,7 @@
 assembly, matrix-free stencil SpMV, moving-PML sweeping preconditioner and preconditioned GMRES, as
 hand-written sm_100a CUDA kernels behind a C ABI (include/helmholtz_b200.h)."""
 from ._lib import HelmholtzB200Error, LIB_PATH, load  # noqa: F401
-from .fields import (init_c1_f1, init_c1_f2, init_c1_mat, init_c2_f1, init_c2_f2, init_c2_mat,  # noqa: F401
+from .fields import (attenuate, init_c1_f1, init_c1_f2, init_c1_mat, init_c2_f1, init_c2_f2, init_c2_mat,  # noqa: F401
                      init_const_f1, init_f1_mat, init_f2_mat, init_layered_f1)
 
 

@@ -21,6 +21,8 @@ SIGNATURES = {
     "hp_profile_enable": (_i, [_vp, _i]),
     "hp_profile_read": (_i, [_vp, C.POINTER(_d), _ip, C.POINTER(_i64)]),
     "hp_create": (_i, [C.POINTER(_vp), _i, _i, _d, _d, _d, _vp, _i, _vp]),
+    "hp_create_complex": (_i, [C.POINTER(_vp), _i, _i, _d, _d, _d, _vp, _i, _vp]),
+    "hp_medium_is_complex": (_i, [_vp]),
     "hp_destroy": (_i, [_vp]),
     "hp_context_clone": (_i, [_vp, C.POINTER(_vp), _vp]),
     "hp_cgs_pass": (_i, [_i, _i64, _i, C.POINTER(_vp), _i64, C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_vp), _i, _i, _vp]),

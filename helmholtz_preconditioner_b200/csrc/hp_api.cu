@@ -62,8 +62,9 @@ extern "C" int hp_device_ok(void) {
     return 1;
 }
 
+// cplx_medium: c_mat holds (n+2)^2 interleaved complex numbers; the solver keeps the complex slowness^2 kappa_c only
 static int hp_create_fill(hp_solver* s, int n, int b, double omega_re, double omega_im, double cst, const double* c_mat,
-                          int c_is_device, cudaStream_t st) {
+                          int c_is_device, int cplx_medium, cudaStream_t st) {
     s->n = n; s->b = b;
     double h = 1.0 / (double)(n + 1);                     // code.py:443
     s->pml.cst = cst; s->pml.h = h; s->pml.eta = (double)b * h;   // code.py:444
@@ -75,35 +76,64 @@ static int hp_create_fill(hp_solver* s, int n, int b, double omega_re, double om
     size_t tl = sizeof(cplx) * (size_t)(2 * n + 3);
     HP_CUDA(cudaMalloc(&s->s1t, tl)); HP_CUDA(cudaMalloc(&s->is1t, tl));
     HP_CUDA(cudaMalloc(&s->s2t, tl)); HP_CUDA(cudaMalloc(&s->is2t, tl));
+    HP_CUDA(cudaMalloc(&s->status, sizeof(int)));
+    HP_CUDA(cudaMemsetAsync(s->status, 0, sizeof(int), st));
+    if (cplx_medium) {
+        // the complex velocity is needed only to form kappa_c: a host model is staged through a temporary device copy
+        const size_t cb = sizeof(cplx) * (size_t)(n + 2) * (n + 2);
+        HP_CUDA(cudaMalloc(&s->kappa_c, sizeof(cplx) * (size_t)n * n));
+        struct Stage { void* p = nullptr; ~Stage() { cudaFree(p); } } stage;
+        const cplx* c_dev = (const cplx*)c_mat;
+        if (!c_is_device) {
+            HP_CUDA(cudaMalloc(&stage.p, cb));
+            HP_CUDA(cudaMemcpyAsync(stage.p, c_mat, cb, cudaMemcpyHostToDevice, st));
+            c_dev = (const cplx*)stage.p;
+        }
+        if (hp_launch_tables(s, c_dev, st)) return 2;
+        s->s2t_h.resize(2 * n + 3);
+        HP_CUDA(cudaMemcpyAsync(s->s2t_h.data(), s->s2t, tl, cudaMemcpyDeviceToHost, st));
+        HP_CUDA(cudaStreamSynchronize(st));                // before the staging copy is freed
+        return 0;
+    }
     size_t cb = sizeof(double) * (size_t)(n + 2) * (n + 2);
     HP_CUDA(cudaMalloc(&s->c_mat, cb));
     HP_CUDA(cudaMalloc(&s->kappa, sizeof(double) * (size_t)n * n));
-    HP_CUDA(cudaMalloc(&s->status, sizeof(int)));
-    HP_CUDA(cudaMemsetAsync(s->status, 0, sizeof(int), st));
     HP_CUDA(cudaMemcpyAsync(s->c_mat, c_mat, cb, c_is_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, st));
-    if (hp_launch_tables(s, st)) return 2;
+    if (hp_launch_tables(s, nullptr, st)) return 2;
     s->s2t_h.resize(2 * n + 3);
     HP_CUDA(cudaMemcpyAsync(s->s2t_h.data(), s->s2t, tl, cudaMemcpyDeviceToHost, st));
     HP_CUDA(cudaStreamSynchronize(st));
     return 0;
 }
 
-extern "C" int hp_create(hp_solver** out, int n, int b, double omega_re, double omega_im, double cst,
-                         const double* c_mat, int c_is_device, void* stream) {
-    if (!out) { hp_set_error("hp_create: null output"); return 1; }
+static int hp_create_any(const char* what, hp_solver** out, int n, int b, double omega_re, double omega_im, double cst,
+                         const double* c_mat, int c_is_device, int cplx_medium, void* stream) {
+    if (!out) { hp_set_error("%s: null output", what); return 1; }
     *out = nullptr;
     if (n < 2 || b < 1 || b > HP_BMAX || b > n) {
-        hp_set_error("hp_create: need 2 <= n, 1 <= b <= min(n, %d); got n=%d b=%d", HP_BMAX, n, b);
+        hp_set_error("%s: need 2 <= n, 1 <= b <= min(n, %d); got n=%d b=%d", what, HP_BMAX, n, b);
         return 1;
     }
-    if (!hp_device_ok()) { hp_set_error("hp_create: no CUDA device (this library has no CPU path)"); return 2; }
+    if (!hp_device_ok()) { hp_set_error("%s: no CUDA device (this library has no CPU path)", what); return 2; }
     cudaStream_t st = (cudaStream_t)stream;
     hp_solver* s = new hp_solver();
-    int rc = hp_create_fill(s, n, b, omega_re, omega_im, cst, c_mat, c_is_device, st);
+    int rc = hp_create_fill(s, n, b, omega_re, omega_im, cst, c_mat, c_is_device, cplx_medium, st);
     if (rc) { hp_destroy(s); return rc; }      // frees whatever was allocated before the failure
     *out = s;
     return 0;
 }
+
+extern "C" int hp_create(hp_solver** out, int n, int b, double omega_re, double omega_im, double cst,
+                         const double* c_mat, int c_is_device, void* stream) {
+    return hp_create_any("hp_create", out, n, b, omega_re, omega_im, cst, c_mat, c_is_device, 0, stream);
+}
+
+extern "C" int hp_create_complex(hp_solver** out, int n, int b, double omega_re, double omega_im, double cst,
+                                 const double* c_mat, int c_is_device, void* stream) {
+    return hp_create_any("hp_create_complex", out, n, b, omega_re, omega_im, cst, c_mat, c_is_device, 1, stream);
+}
+
+extern "C" int hp_medium_is_complex(hp_solver* s) { return s && s->kappa_c ? 1 : 0; }
 
 // A second handle on the same operator and factorisation with its own sweep scratch (exchange ring, abort flags, parked
 // front solutions): sweeps issued through different contexts may be in flight on different streams at the same time
@@ -160,7 +190,7 @@ extern "C" int hp_destroy(hp_solver* s) {
     }
     hp_free_strips(s);
     cudaFree(s->s1t); cudaFree(s->is1t); cudaFree(s->s2t); cudaFree(s->is2t);
-    cudaFree(s->c_mat); cudaFree(s->kappa); cudaFree(s->status);
+    cudaFree(s->c_mat); cudaFree(s->kappa); cudaFree(s->kappa_c); cudaFree(s->status);
     cudaFree(s->f_low); cudaFree(s->f_invd); cudaFree(s->f_up); cudaFree(s->TF); cudaFree(s->TFm);
     hp_front_coupled_free(s);
     for (cudaEvent_t e : s->prof_ev) cudaEventDestroy(e);

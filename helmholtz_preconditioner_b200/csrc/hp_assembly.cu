@@ -8,7 +8,9 @@
 //     c5 = omega^2/(s1 s2 c^2) - (c1+c2+c3+c4),
 // so the stretching factors are evaluated once per grid line (2n+3 half-grid points per axis, kernel
 // hp_tables_kernel) and the per-point work is a handful of complex multiplies: both kernels below are
-// HBM-bound (CSR: 104 B written per row; matvec: 40 B per grid point).
+// HBM-bound (CSR: 104 B written per row; matvec: 40 B per grid point, 48 B for an attenuating medium).
+// The kernels that read the slowness^2 kappa = 1/c^2 are templates on its type: double for a real medium, cplx for an
+// attenuating one (hp_create_complex); the real instances are the code of the real-only kernels.
 #include "hp_internal.cuh"
 #include <stdlib.h>
 
@@ -36,21 +38,43 @@ __global__ void hp_kappa_kernel(int n, const double* __restrict__ c_mat, double*
     }
 }
 
-int hp_launch_tables(hp_solver* s, cudaStream_t st) {
+// the same for an attenuating medium: kappa_c = 1/(c*c) with the complex multiply and Smith's division of hp_small.h, so
+// that c = (cr, 0) gives (1/cr^2, 0) bit for bit.  c_mat is (n+2)^2 interleaved complex.
+__global__ void hp_kappa_c_kernel(int n, const cplx* __restrict__ c_mat, cplx* __restrict__ kappa_c) {
+    __shared__ cplx tile[32][33];
+    int i0 = blockIdx.x * 32, j0 = blockIdx.y * 32;
+    for (int r = threadIdx.y; r < 32; r += blockDim.y) {
+        int i = i0 + r, j = j0 + threadIdx.x;
+        if (i < n && j < n) tile[r][threadIdx.x] = c_mat[(size_t)i * (n + 2) + j];
+    }
+    __syncthreads();
+    for (int r = threadIdx.y; r < 32; r += blockDim.y) {
+        int j = j0 + r, i = i0 + threadIdx.x;
+        if (i < n && j < n) {
+            cplx c = tile[threadIdx.x][r];
+            kappa_c[(size_t)j * n + i] = cinv(cmul(c, c));
+        }
+    }
+}
+
+// c_cplx: the (n+2)^2 complex velocity on the device for an attenuating medium (s->kappa_c set), unused otherwise
+int hp_launch_tables(hp_solver* s, const cplx* c_cplx, cudaStream_t st) {
     int n = s->n, len = 2 * n + 3;
     hp_count_launch(); hp_tables_kernel<<<(len + 127) / 128, 128, 0, st>>>(n, s->pml, s->s1t, s->is1t, s->s2t, s->is2t);
     dim3 blk(32, 8), grd((n + 31) / 32, (n + 31) / 32);
-    hp_count_launch(); hp_kappa_kernel<<<grd, blk, 0, st>>>(n, s->c_mat, s->kappa);
+    if (s->kappa_c) { hp_count_launch(); hp_kappa_c_kernel<<<grd, blk, 0, st>>>(n, c_cplx, s->kappa_c); }
+    else { hp_count_launch(); hp_kappa_kernel<<<grd, blk, 0, st>>>(n, s->c_mat, s->kappa); }
     HP_CUDA(cudaGetLastError());
     return 0;
 }
 
 struct HpPointCoef { cplx c1, c2, c3, c4, c5; };
 
+template <typename KT>
 __device__ __forceinline__ HpPointCoef hp_point_coef(int i, int j, int n, double ih2, cplx omega2,
                                                      const cplx* __restrict__ s1t, const cplx* __restrict__ is1t,
                                                      const cplx* __restrict__ s2t, const cplx* __restrict__ is2t,
-                                                     double kap) {
+                                                     KT kap) {
     // i, j are 1-based grid indices
     cplx is2c = is2t[2 * j], is1c = is1t[2 * i];
     HpPointCoef c;
@@ -58,8 +82,7 @@ __device__ __forceinline__ HpPointCoef hp_point_coef(int i, int j, int n, double
     c.c2 = cscale(ih2, cmul(s1t[2 * i + 1], is2c));
     c.c3 = cscale(ih2, cmul(s2t[2 * j - 1], is1c));
     c.c4 = cscale(ih2, cmul(s2t[2 * j + 1], is1c));
-    cplx t = cscale(kap, cmul(omega2, cmul(is1c, is2c)));
-    c.c5 = csub(t, cadd(cadd(c.c1, c.c2), cadd(c.c3, c.c4)));
+    c.c5 = hp_kmul_sub(kap, cmul(omega2, cmul(is1c, is2c)), cadd(cadd(c.c1, c.c2), cadd(c.c3, c.c4)));
     return c;
 }
 
@@ -73,9 +96,10 @@ __device__ __forceinline__ int64_t hp_csr_row_offset(int64_t r, int64_t nn) {
     const int64_t j0 = r / nn, i0 = r - j0 * nn;
     return 5 * r - (r < nn ? r : nn) - (r > (nn - 1) * nn ? r - (nn - 1) * nn : 0) - (j0 + (i0 > 0 ? 1 : 0)) - j0;
 }
+template <typename KT>
 __global__ void __launch_bounds__(HP_ASM_THREADS) hp_assemble_csr_kernel(int n, double ih2, cplx omega2,
         const cplx* __restrict__ s1t, const cplx* __restrict__ is1t, const cplx* __restrict__ s2t,
-        const cplx* __restrict__ is2t, const double* __restrict__ kappa,
+        const cplx* __restrict__ is2t, const KT* __restrict__ kappa,
         int32_t* __restrict__ indptr, int32_t* __restrict__ indices, cplx* __restrict__ data) {
     __shared__ cplx sdata[HP_ASM_THREADS * 5];
     __shared__ int32_t sidx[HP_ASM_THREADS * 5];
@@ -114,6 +138,7 @@ __device__ __forceinline__ int64_t hp_strip_row_offset(int64_t r, int64_t nn, in
     const int64_t k0 = r / nn, i0 = r - k0 * nn;
     return 5 * r - (r < nn ? r : nn) - (r > (b - 1) * nn ? r - (b - 1) * nn : 0) - (k0 + (i0 > 0 ? 1 : 0)) - k0;
 }
+template <bool CK>
 __global__ void hp_strip_csr_kernel(HpStripCtx c, int m, int32_t* __restrict__ indptr, int32_t* __restrict__ indices,
                                     cplx* __restrict__ data) {
     const int i0 = blockIdx.x * blockDim.x + threadIdx.x;       // 0-based column
@@ -122,7 +147,7 @@ __global__ void hp_strip_csr_kernel(HpStripCtx c, int m, int32_t* __restrict__ i
     HpStripRow R;
     hp_strip_rows(R, m, b, c.pml);
     HpBlockRow B;
-    hp_block_row(B, R, i0 + 1, m, b, n, c.pml, c.s1t, c.is1t, c.c_mat, c.omega2);
+    hp_block_row<CK>(B, R, i0 + 1, m, b, n, c.pml, c.s1t, c.is1t, c.c_mat, c.omega2, c.kappa_c);
     for (int k = 0; k < b; ++k) {
         const int64_t r = (int64_t)k * n + i0;
         int64_t o = hp_strip_row_offset(r, n, b);
@@ -140,7 +165,8 @@ extern "C" int hp_assemble_strip_csr(hp_solver* s, int m, int32_t* indptr_dev, i
     if (!s) { hp_set_error("hp_assemble_strip_csr: null solver"); return 1; }
     if (m < s->b || m > s->n) { hp_set_error("hp_assemble_strip_csr: layer m must lie in %d..%d, got %d", s->b, s->n, m); return 1; }
     hp_count_launch();
-    hp_strip_csr_kernel<<<(s->n + 63) / 64, 64, 0, (cudaStream_t)stream>>>(hp_ctx(s), m, indptr_dev, indices_dev, (cplx*)data_dev);
+    if (s->kappa_c) hp_strip_csr_kernel<true><<<(s->n + 63) / 64, 64, 0, (cudaStream_t)stream>>>(hp_ctx(s), m, indptr_dev, indices_dev, (cplx*)data_dev);
+    else hp_strip_csr_kernel<false><<<(s->n + 63) / 64, 64, 0, (cudaStream_t)stream>>>(hp_ctx(s), m, indptr_dev, indices_dev, (cplx*)data_dev);
     HP_CUDA(cudaGetLastError());
     return 0;
 }
@@ -149,16 +175,17 @@ extern "C" int hp_assemble_strip_csr(hp_solver* s, int m, int32_t* indptr_dev, i
 // each thread keeps the x2 neighbours (south, centre, north) of its column in registers, takes the x1
 // neighbours from the adjacent lanes by shuffle (warp-edge lanes read them from L1/L2) and keeps the
 // x1-dependent factors in registers for the whole march.  Algorithmic traffic per grid point:
-// x 16 B read + y 16 B written + kappa 8 B read = 40 B.
+// x 16 B read + y 16 B written + kappa 8 B read = 40 B (48 B with the complex kappa of an attenuating medium).
 // The march length (rows per CTA) is chosen by the host so that the whole grid is ONE wave of resident CTAs
 // (hp_spmv_rows): with a fixed 16 rows the 8192 CTAs of 4096^2 ran as 6.9 waves of 1184 and the last, partly filled
 // wave cost 7 % of the kernel; longer marches also read fewer halo rows twice (2 per march).
 #define HP_SPMV_MIN_ROWS 16
 // Rows j_lo <= j < j_hi (0-based) of the grid: x and y hold those rows only (slab storage); the rows just
 // outside come from the halo pointers x_south (row j_lo-1) and x_north (row j_hi), NULL on the grid boundary.
+template <typename KT>
 __global__ void __launch_bounds__(128) hp_stencil_matvec_kernel(int n, int j_lo, int j_hi, int rows, int pf, double ih2, cplx omega2,
         const cplx* __restrict__ s1t, const cplx* __restrict__ is1t, const cplx* __restrict__ s2t,
-        const cplx* __restrict__ is2t, const double* __restrict__ kappa,
+        const cplx* __restrict__ is2t, const KT* __restrict__ kappa,
         const cplx* __restrict__ x, const cplx* __restrict__ x_south, const cplx* __restrict__ x_north,
         cplx* __restrict__ y) {
     const int col = blockIdx.x * 128 + threadIdx.x;
@@ -189,14 +216,16 @@ __global__ void __launch_bounds__(128) hp_stencil_matvec_kernel(int n, int j_lo,
         if (pf > 0 && threadIdx.x == 0 && j + pf < j1) {
             if (j + pf + 1 < j_hi)
                 asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(x + base + (size_t)(pf + 1) * n + blockIdx.x * 128), "r"(pcols * 16) : "memory");
-            if ((n & 1) == 0) asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(kappa + (size_t)(j + pf) * n + blockIdx.x * 128), "r"(pcols * 8) : "memory");
+            // a bulk prefetch wants 16-byte aligned rows: always so for a complex kappa, for n even for a real one
+            if (sizeof(KT) == 16 || (n & 1) == 0)
+                asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(kappa + (size_t)(j + pf) * n + blockIdx.x * 128), "r"(pcols * (int)sizeof(KT)) : "memory");
         }
         cplx xN = zero;
         if (act) {
             if (j + 1 < j_hi) xN = x[base + n + col];
             else if (x_north) xN = x_north[col];
         }
-        double kap = act ? kappa[(size_t)j * n + col] : 0.0;
+        KT kap = act ? kappa[(size_t)j * n + col] : KT{};
         cplx xW, xE;
         xW.x = __shfl_up_sync(0xffffffffu, xC.x, 1);
         xW.y = __shfl_up_sync(0xffffffffu, xC.y, 1);
@@ -210,7 +239,7 @@ __global__ void __launch_bounds__(128) hp_stencil_matvec_kernel(int n, int j_lo,
         // y = c5 xC + c1 xW + c2 xE + c3 xS + c4 xN with c5 = kappa omega^2 dI bJ - (c1+c2+c3+c4)
         cplx t1 = cfma(aW, csub(xW, xC), cmul(aE, csub(xE, xC)));
         cplx t2 = cfma(gS, csub(xS, xC), cmul(gN, csub(xN, xC)));
-        cplx acc = cmul(cscale(kap, cmul(wI, bJ)), xC);
+        cplx acc = cmul(hp_kmul(kap, cmul(wI, bJ)), xC);
         acc = cfma(bJ, t1, acc);
         acc = cfma(dI, t2, acc);
         if (act) y[base + col] = acc;
@@ -236,8 +265,12 @@ extern "C" int hp_assemble_csr(hp_solver* s, int32_t* indptr, int32_t* indices, 
     if (hp_csr_nnz(s->n) > 2147483647LL) { hp_set_error("hp_assemble_csr: nnz exceeds int32 indices"); return 1; }
     int64_t N = (int64_t)s->n * s->n;
     double ih2 = 1.0 / (s->pml.h * s->pml.h);
-    hp_count_launch(); hp_assemble_csr_kernel<<<(unsigned)((N + HP_ASM_THREADS - 1) / HP_ASM_THREADS), HP_ASM_THREADS, 0, (cudaStream_t)stream>>>(
-        s->n, ih2, s->omega2, s->s1t, s->is1t, s->s2t, s->is2t, s->kappa, indptr, indices, (cplx*)data);
+    const unsigned grd = (unsigned)((N + HP_ASM_THREADS - 1) / HP_ASM_THREADS);
+    hp_count_launch();
+    if (s->kappa_c) hp_assemble_csr_kernel<<<grd, HP_ASM_THREADS, 0, (cudaStream_t)stream>>>(
+        s->n, ih2, s->omega2, s->s1t, s->is1t, s->s2t, s->is2t, (const cplx*)s->kappa_c, indptr, indices, (cplx*)data);
+    else hp_assemble_csr_kernel<<<grd, HP_ASM_THREADS, 0, (cudaStream_t)stream>>>(
+        s->n, ih2, s->omega2, s->s1t, s->is1t, s->s2t, s->is2t, (const double*)s->kappa, indptr, indices, (cplx*)data);
     HP_CUDA(cudaGetLastError());
     return 0;
 }
@@ -250,7 +283,7 @@ static int hp_spmv_rows(int n, int nrows) {
     if (!slots) {
         int dev = 0, sms = 0, per_sm = 0;
         if (cudaGetDevice(&dev) == cudaSuccess && cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) == cudaSuccess &&
-            cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, hp_stencil_matvec_kernel, 128, 0) == cudaSuccess && per_sm > 0)
+            cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, hp_stencil_matvec_kernel<double>, 128, 0) == cudaSuccess && per_sm > 0)
             slots = sms * per_sm;
         else { cudaGetLastError(); slots = 1184; }
     }
@@ -273,8 +306,12 @@ extern "C" int hp_stencil_matvec_rows(hp_solver* s, int j_lo, int j_hi, const do
     double ih2 = 1.0 / (s->pml.h * s->pml.h);
     const int rows = hp_spmv_rows(s->n, j_hi - j_lo);
     dim3 grd((s->n + 127) / 128, (j_hi - j_lo + rows - 1) / rows);
-    hp_count_launch(); hp_stencil_matvec_kernel<<<grd, 128, 0, (cudaStream_t)stream>>>(
-        s->n, j_lo, j_hi, rows, hp_spmv_pf(), ih2, s->omega2, s->s1t, s->is1t, s->s2t, s->is2t, s->kappa, (const cplx*)x,
+    hp_count_launch();
+    if (s->kappa_c) hp_stencil_matvec_kernel<<<grd, 128, 0, (cudaStream_t)stream>>>(
+        s->n, j_lo, j_hi, rows, hp_spmv_pf(), ih2, s->omega2, s->s1t, s->is1t, s->s2t, s->is2t, (const cplx*)s->kappa_c, (const cplx*)x,
+        (const cplx*)x_south, (const cplx*)x_north, (cplx*)y);
+    else hp_stencil_matvec_kernel<<<grd, 128, 0, (cudaStream_t)stream>>>(
+        s->n, j_lo, j_hi, rows, hp_spmv_pf(), ih2, s->omega2, s->s1t, s->is1t, s->s2t, s->is2t, (const double*)s->kappa, (const cplx*)x,
         (const cplx*)x_south, (const cplx*)x_north, (cplx*)y);
     HP_CUDA(cudaGetLastError());
     return 0;

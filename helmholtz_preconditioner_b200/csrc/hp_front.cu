@@ -6,10 +6,12 @@
 // (code.py:364-365 and 381-384).  Here: Thomas factors computed once, one thread per grid row.
 #include "hp_internal.cuh"
 
-// factors stored [i][j] (x1 index major) so that the b threads of the solve read contiguous memory
+// factors stored [i][j] (x1 index major) so that the b threads of the solve read contiguous memory.  KT: double for a real
+// medium, cplx for an attenuating one (see hp_kmul)
+template <typename KT>
 __global__ void hp_front_factor_kernel(int n, int b, double ih2, cplx omega2, const cplx* __restrict__ s1t,
                                        const cplx* __restrict__ is1t, const cplx* __restrict__ s2t,
-                                       const cplx* __restrict__ is2t, const double* __restrict__ kappa,
+                                       const cplx* __restrict__ is2t, const KT* __restrict__ kappa,
                                        cplx* __restrict__ low, cplx* __restrict__ invd, cplx* __restrict__ up,
                                        int* status) {
     int j0 = threadIdx.x;            // 0-based grid row
@@ -23,8 +25,7 @@ __global__ void hp_front_factor_kernel(int n, int b, double ih2, cplx omega2, co
         cplx c1 = cscale(ih2, cmul(s1t[2 * i - 1], is2c));
         cplx c2 = cscale(ih2, cmul(s1t[2 * i + 1], is2c));
         cplx c3 = cmul(g3, is1c), c4 = cmul(g4, is1c);
-        cplx c5 = cscale(kappa[(size_t)j0 * n + (i - 1)], cmul(omega2, cmul(is1c, is2c)));
-        c5 = csub(c5, cadd(cadd(c1, c2), cadd(c3, c4)));
+        cplx c5 = hp_kmul_sub(kappa[(size_t)j0 * n + (i - 1)], cmul(omega2, cmul(is1c, is2c)), cadd(cadd(c1, c2), cadd(c3, c4)));
         cplx w = cmake(0.0, 0.0), d = c5;
         if (i > 1) {
             w = cdiv(c1, dprev);
@@ -238,8 +239,11 @@ int hp_front_setup(hp_solver* s, cudaStream_t st) {
         HP_CUDA(cudaMalloc(&s->TF, sz + sizeof(cplx) * (size_t)s->b * s->n));   // TF followed by the work rows
     }
     double ih2 = 1.0 / (s->pml.h * s->pml.h);
-    hp_count_launch(); hp_front_factor_kernel<<<1, 32, 0, st>>>(s->n, s->b, ih2, s->omega2, s->s1t, s->is1t, s->s2t, s->is2t, s->kappa,
-                                             s->f_low, s->f_invd, s->f_up, s->status);
+    hp_count_launch();
+    if (s->kappa_c) hp_front_factor_kernel<<<1, 32, 0, st>>>(s->n, s->b, ih2, s->omega2, s->s1t, s->is1t, s->s2t, s->is2t,
+                                                             (const cplx*)s->kappa_c, s->f_low, s->f_invd, s->f_up, s->status);
+    else hp_front_factor_kernel<<<1, 32, 0, st>>>(s->n, s->b, ih2, s->omega2, s->s1t, s->is1t, s->s2t, s->is2t,
+                                                  (const double*)s->kappa, s->f_low, s->f_invd, s->f_up, s->status);
     HP_CUDA(cudaGetLastError());
     if (s->front_mode == 1) return hp_front_coupled_setup(s, st);
     hp_front_coupled_free(s);

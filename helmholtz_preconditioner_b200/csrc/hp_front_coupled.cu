@@ -173,20 +173,22 @@ __global__ void __launch_bounds__(32) hp_fc_schur_solve_kernel(HpFcArgs a, int r
 
 // ---- setup -------------------------------------------------------------------------------------------------------
 // thread -> leaf: forward Schur chain of the leaf (the strip arithmetic of csrc/hp_setup_core.h with m = b)
-template <int BB>
+// (CK: attenuating medium, hp_block_row)
+template <int BB, bool CK>
 __global__ void hp_fc_chain_kernel(HpStripCtx c, int P, const int* leaf_start, const int* leaf_q, cplx* Sinv, int* status) {
     const int l = blockIdx.x * blockDim.x + threadIdx.x;
     if (l >= P) return;
-    if (hp_chain_forward<BB>(Sinv, leaf_start[l] + 1, leaf_start[l] + leaf_q[l], c.b, c)) atomicOr(status, 16);
+    if (hp_chain_forward<BB, CK>(Sinv, leaf_start[l] + 1, leaf_start[l] + leaf_q[l], c.b, c)) atomicOr(status, 16);
 }
 // thread -> grid column: the x1 couplings and the tridiagonal block D_i of every column
+template <bool CK>
 __global__ void hp_fc_coef_kernel(HpStripCtx c, cplx* LU, cplx* D3) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;      // 0-based column
     if (i >= c.n) return;
     HpStripRow R;
     hp_strip_rows(R, c.b, c.b, c.pml);
     HpBlockRow B;
-    hp_block_row(B, R, i + 1, c.b, c.b, c.n, c.pml, c.s1t, c.is1t, c.c_mat, c.omega2);
+    hp_block_row<CK>(B, R, i + 1, c.b, c.b, c.n, c.pml, c.s1t, c.is1t, c.c_mat, c.omega2, c.kappa_c);
     for (int k = 0; k < c.b; ++k) {
         LU[((size_t)i * 2) * c.b + k] = B.L[k];
         LU[((size_t)i * 2 + 1) * c.b + k] = B.U[k];
@@ -331,9 +333,16 @@ int hp_front_coupled_setup(hp_solver* s, cudaStream_t st) {
     HP_CUDA(cudaMalloc(&corners, sizeof(cplx) * (size_t)P * 2 * b * 2 * b));
     HpStripCtx c = hp_ctx(s);
     hp_count_launch();
-    if (b <= 12) hp_fc_chain_kernel<144><<<(P + 31) / 32, 32, 0, st>>>(c, P, s->fc_leaf_start, s->fc_leaf_q, s->fc_Sinv, s->status);
-    else hp_fc_chain_kernel<HP_BMAX * HP_BMAX><<<(P + 31) / 32, 32, 0, st>>>(c, P, s->fc_leaf_start, s->fc_leaf_q, s->fc_Sinv, s->status);
-    hp_count_launch(); hp_fc_coef_kernel<<<(n + 63) / 64, 64, 0, st>>>(c, s->fc_LU, D3);
+    const bool ck = s->kappa_c != nullptr;
+    if (ck) {
+        if (b <= 12) hp_fc_chain_kernel<144, true><<<(P + 31) / 32, 32, 0, st>>>(c, P, s->fc_leaf_start, s->fc_leaf_q, s->fc_Sinv, s->status);
+        else hp_fc_chain_kernel<HP_BMAX * HP_BMAX, true><<<(P + 31) / 32, 32, 0, st>>>(c, P, s->fc_leaf_start, s->fc_leaf_q, s->fc_Sinv, s->status);
+        hp_count_launch(); hp_fc_coef_kernel<true><<<(n + 63) / 64, 64, 0, st>>>(c, s->fc_LU, D3);
+    } else {
+        if (b <= 12) hp_fc_chain_kernel<144, false><<<(P + 31) / 32, 32, 0, st>>>(c, P, s->fc_leaf_start, s->fc_leaf_q, s->fc_Sinv, s->status);
+        else hp_fc_chain_kernel<HP_BMAX * HP_BMAX, false><<<(P + 31) / 32, 32, 0, st>>>(c, P, s->fc_leaf_start, s->fc_leaf_q, s->fc_Sinv, s->status);
+        hp_count_launch(); hp_fc_coef_kernel<false><<<(n + 63) / 64, 64, 0, st>>>(c, s->fc_LU, D3);
+    }
     HP_CUDA(cudaGetLastError());
     if (ns > 0) {
         if (fc_leaf(s, 2 * b, 1, 0, 1, nullptr, nullptr, corners, nullptr, cmake(0, 0), st)) return 2;

@@ -53,8 +53,9 @@ struct hp_solver {
     // operator tables on the half grid t = 0..2n+2 (unshifted PML)
     cplx *s1t = nullptr, *is1t = nullptr, *s2t = nullptr, *is2t = nullptr;
     std::vector<cplx> s2t_h;      // host copy of s2t (couplings between grid rows are formed on the host)
-    double* c_mat = nullptr;      // (n+2)^2 as given
-    double* kappa = nullptr;      // n*n, kappa[(j-1)*n + (i-1)] = 1 / c_mat[i-1][j-1]^2  (grid-aligned)
+    double* c_mat = nullptr;      // (n+2)^2 as given (real medium)
+    double* kappa = nullptr;      // n*n, kappa[(j-1)*n + (i-1)] = 1 / c_mat[i-1][j-1]^2  (grid-aligned, real medium)
+    cplx* kappa_c = nullptr;      // attenuating medium (hp_create_complex): the same n*n array, complex; c_mat and kappa stay NULL
     // strip factorisation
     HpLayout lay;
     int m_lo = 0, m_hi = -1;      // strips held by this solver
@@ -100,12 +101,12 @@ struct hp_solver {
 static inline HpStripCtx hp_ctx(const hp_solver* s) {
     HpStripCtx c;
     c.n = s->n; c.b = s->b; c.pml = s->pml; c.omega2 = s->omega2;
-    c.s1t = s->s1t; c.is1t = s->is1t; c.c_mat = s->c_mat;
+    c.s1t = s->s1t; c.is1t = s->is1t; c.c_mat = s->c_mat; c.kappa_c = s->kappa_c;
     return c;
 }
 
 // hp_assembly.cu
-int hp_launch_tables(hp_solver* s, cudaStream_t st);
+int hp_launch_tables(hp_solver* s, const cplx* c_cplx, cudaStream_t st);   // c_cplx: complex velocity (attenuating medium) or NULL
 // hp_setup.cu
 int hp_setup_strips(hp_solver* s, int P, int K, int m_lo, int m_hi, cudaStream_t st);
 void hp_free_strips(hp_solver* s);

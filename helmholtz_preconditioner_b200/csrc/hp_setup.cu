@@ -63,6 +63,7 @@ __device__ __forceinline__ HpLaneRow hp_lane_strip_row(int k, int m, int b, cons
     return R;
 }
 // coefficients of block row i for strip row k (cf. hp_block_row): written to vec[0..5b) = L, U, sub, dia, sup
+template <bool CK>
 __device__ __forceinline__ void hp_lane_block_row(cplx* vec, const HpLaneRow& R, int i, int k, int m, int b, const HpStripCtx& c) {
     double ih2 = 1.0 / (c.pml.h * c.pml.h);
     cplx s1lo = c.s1t[2 * i - 1], s1hi = c.s1t[2 * i + 1], is1c = c.is1t[2 * i];
@@ -71,9 +72,15 @@ __device__ __forceinline__ void hp_lane_block_row(cplx* vec, const HpLaneRow& R,
     cplx c2 = cscale(ih2, cmul(s1hi, R.is2c));
     cplx c3 = cscale(ih2, cmul(R.s2lo, is1c));
     cplx c4 = cscale(ih2, cmul(R.s2hi, is1c));
-    double cv = c.c_mat[(size_t)(i - 1) * (c.n + 2) + (j - 1)];
-    cplx c5 = cscale(1.0 / (cv * cv), cmul(c.omega2, cmul(is1c, R.is2c)));
-    c5 = csub(c5, cadd(cadd(c1, c2), cadd(c3, c4)));
+    cplx c5;
+    if constexpr (CK) {
+        c5 = hp_kmul_sub(c.kappa_c[(size_t)(j - 1) * c.n + (i - 1)], cmul(c.omega2, cmul(is1c, R.is2c)),
+                         cadd(cadd(c1, c2), cadd(c3, c4)));
+    } else {
+        double cv = c.c_mat[(size_t)(i - 1) * (c.n + 2) + (j - 1)];
+        c5 = cscale(1.0 / (cv * cv), cmul(c.omega2, cmul(is1c, R.is2c)));
+        c5 = csub(c5, cadd(cadd(c1, c2), cadd(c3, c4)));
+    }
     vec[k] = c1; vec[b + k] = c2; vec[2 * b + k] = c3; vec[3 * b + k] = c5; vec[4 * b + k] = c4;
 }
 // in-place Gauss-Jordan inverse with partial pivoting of the b x b matrix A in shared memory (b <= 32), one warp.
@@ -122,6 +129,7 @@ __device__ int hp_warp_inv(cplx* A, int b, int lane, int* piv) {
     return bad;
 }
 
+template <bool CK>
 __global__ void __launch_bounds__(256) hp_chain_warp_kernel(HpSetupArgs a, int warps_per_block) {
     extern __shared__ double2 smw[];
     const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
@@ -145,7 +153,7 @@ __global__ void __launch_bounds__(256) hp_chain_warp_kernel(HpSetupArgs a, int w
     const int nsteps = i1 - i0 + 1;
     for (int st = 0; st < nsteps; ++st) {
         const int i = dir == 0 ? i0 + st : i1 - st;
-        if (lane < b) hp_lane_block_row(vec, R, i, lane, m, b, a.c);
+        if (lane < b) hp_lane_block_row<CK>(vec, R, i, lane, m, b, a.c);
         __syncwarp();
         // F = D_i - diag(a) Xinv diag(c):  forward a = L_i, c = U_{i-1};  backward a = U_i, c = L_{i+1}
         const cplx* av = dir == 0 ? vec : vec + b;
@@ -170,7 +178,7 @@ __global__ void __launch_bounds__(256) hp_chain_warp_kernel(HpSetupArgs a, int w
         cplx* G = F;
         cplx* gcol = a.gcol + (size_t)lb * n * b;
         for (int i = i0; i <= i1; ++i) {
-            if (lane < b) hp_lane_block_row(vec, R, i, lane, m, b, a.c);
+            if (lane < b) hp_lane_block_row<CK>(vec, R, i, lane, m, b, a.c);
             __syncwarp();
             if (i > i0) {
                 const cplx* Bi = out + (size_t)(i - 1) * bb;
@@ -324,7 +332,7 @@ __device__ __forceinline__ int hp_half_inv(cplx (&A)[B], int j) {
     }
 }
 
-template <int B, bool ROLL>
+template <int B, bool ROLL, bool CK = false>
 __global__ void __launch_bounds__(128, 4) hp_chain_reg_kernel(HpSetupArgs a) {
     constexpr int BBc = B * B, RH = (B + 1) / 2;
     __shared__ cplx s_tab[4][B];                 // 1/s2 at the strip rows (both halves work on the same strip)
@@ -354,9 +362,14 @@ __global__ void __launch_bounds__(128, 4) hp_chain_reg_kernel(HpSetupArgs a) {
         c2 = cscale(ih2, cmul(s1hi, Rj.is2c));
         const cplx c3 = cscale(ih2, cmul(Rj.s2lo, is1c));
         const cplx c4 = cscale(ih2, cmul(Rj.s2hi, is1c));
-        const double cv = a.c.c_mat[(size_t)(i - 1) * (n + 2) + (jg - 1)];
-        const cplx c5 = cscale(1.0 / (cv * cv), cmul(a.c.omega2, cmul(is1c, Rj.is2c)));
-        dia = csub(c5, cadd(cadd(c1, c2), cadd(c3, c4)));
+        if constexpr (CK) {
+            dia = hp_kmul_sub(a.c.kappa_c[(size_t)(jg - 1) * n + (i - 1)], cmul(a.c.omega2, cmul(is1c, Rj.is2c)),
+                              cadd(cadd(c1, c2), cadd(c3, c4)));
+        } else {
+            const double cv = a.c.c_mat[(size_t)(i - 1) * (n + 2) + (jg - 1)];
+            const cplx c5 = cscale(1.0 / (cv * cv), cmul(a.c.omega2, cmul(is1c, Rj.is2c)));
+            dia = csub(c5, cadd(cadd(c1, c2), cadd(c3, c4)));
+        }
     };
 
     cplx A[B];
@@ -710,6 +723,7 @@ __global__ void __launch_bounds__(128) hp_corner_kernel(HpSetupArgs a) {
 }
 
 // thread -> (strip, separator)
+template <bool CK>
 __global__ void __launch_bounds__(128) hp_sep_blocks_kernel(HpSetupArgs a) {
     int t = blockIdx.x * blockDim.x + threadIdx.x;
     int ns = a.lay.P - 1, b = a.c.b, bb = b * b, n = a.c.n;
@@ -718,7 +732,7 @@ __global__ void __launch_bounds__(128) hp_sep_blocks_kernel(HpSetupArgs a) {
     int s = a.sep[j] + 1;
     const cplx* Finv = a.Finv + (size_t)lb * n * bb;
     const cplx* Binv = a.Binv + (size_t)lb * n * bb;
-    hp_sep_diag(a.Sd + ((size_t)lb * ns + j) * bb, s, m, Finv + (size_t)(s - 2) * bb, Binv + (size_t)s * bb, a.c);
+    hp_sep_diag<CK>(a.Sd + ((size_t)lb * ns + j) * bb, s, m, Finv + (size_t)(s - 2) * bb, Binv + (size_t)s * bb, a.c);
     if (j + 1 < ns)
         hp_sep_offdiag(a.So + ((size_t)lb * ns + j) * bb, s, a.sep[j + 1] + 1, m,
                        a.tp + ((size_t)lb * a.lay.P + j + 1) * bb, a.c);
@@ -1235,6 +1249,11 @@ struct HpTrace {
 int hp_setup_strips(hp_solver* s, int P_req, int K_req, int m_lo, int m_hi, cudaStream_t st) {
     HpTrace tr;
     const int n = s->n, b = s->b, bb = b * b;
+    const bool ck = s->kappa_c != nullptr;                 // attenuating medium: the complex-kappa instances of the chains
+    if (ck && (getenv("HP_CHAIN_THREAD") || getenv("HP_CHAIN_UNROLL"))) {
+        hp_set_error("hp_precond_setup: the setup generations selected by HP_CHAIN_THREAD / HP_CHAIN_UNROLL support real media only");
+        return 1;
+    }
     hp_free_strips(s);
     const int nstrips = m_hi - m_lo + 1;
     HpLayout L;
@@ -1325,7 +1344,8 @@ int hp_setup_strips(hp_solver* s, int P_req, int K_req, int m_lo, int m_hi, cuda
     if (getenv("HP_CHAIN_THREAD")) chain_wpb = 0;          // developer switch: the one-thread-per-chain kernel
     const size_t chain_smem = chain_per_warp * (size_t)std::max(chain_wpb, 1);
     if (chain_wpb > 0 && chain_smem > 48 * 1024)
-        HP_CUDA(cudaFuncSetAttribute(hp_chain_warp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)chain_smem));
+        HP_CUDA(cudaFuncSetAttribute(ck ? hp_chain_warp_kernel<true> : hp_chain_warp_kernel<false>,
+                                     cudaFuncAttributeMaxDynamicSharedMemorySize, (int)chain_smem));
     for (int m0 = m_lo; m0 <= m_hi; m0 += LB) {
         a.m0 = m0;
         a.nb = std::min(LB, m_hi - m0 + 1);
@@ -1333,9 +1353,11 @@ int hp_setup_strips(hp_solver* s, int P_req, int K_req, int m_lo, int m_hi, cuda
         hp_count_launch();
         if (chain_wpb > 0 && b == 12 && !getenv("HP_CHAIN_SMEM")) {
             if (getenv("HP_CHAIN_UNROLL")) hp_chain_reg_kernel<12, false><<<(a.nb * P + 3) / 4, 128, 0, st>>>(a);
+            else if (ck) hp_chain_reg_kernel<12, true, true><<<(a.nb * P + 3) / 4, 128, 0, st>>>(a);
             else hp_chain_reg_kernel<12, true><<<(a.nb * P + 3) / 4, 128, 0, st>>>(a);        // one warp per leaf: both chains
         } else if (chain_wpb > 0) {
-            hp_chain_warp_kernel<<<(t1 + chain_wpb - 1) / chain_wpb, 32 * chain_wpb, chain_smem, st>>>(a, chain_wpb);
+            if (ck) hp_chain_warp_kernel<true><<<(t1 + chain_wpb - 1) / chain_wpb, 32 * chain_wpb, chain_smem, st>>>(a, chain_wpb);
+            else hp_chain_warp_kernel<false><<<(t1 + chain_wpb - 1) / chain_wpb, 32 * chain_wpb, chain_smem, st>>>(a, chain_wpb);
         } else if (small_b) hp_chain_kernel<144><<<(t1 + 63) / 64, 64, 0, st>>>(a);
         else hp_chain_kernel<HP_BMAX * HP_BMAX><<<(t1 + 63) / 64, 64, 0, st>>>(a);
         hp_count_launch();
@@ -1352,7 +1374,9 @@ int hp_setup_strips(hp_solver* s, int P_req, int K_req, int m_lo, int m_hi, cuda
                 else hp_corner_kernel<<<(t3 + 127) / 128, 128, 0, st>>>(a);
             }
             int t4 = a.nb * ns;
-            hp_count_launch(); hp_sep_blocks_kernel<<<(t4 + 127) / 128, 128, 0, st>>>(a);
+            hp_count_launch();
+            if (ck) hp_sep_blocks_kernel<true><<<(t4 + 127) / 128, 128, 0, st>>>(a);
+            else hp_sep_blocks_kernel<false><<<(t4 + 127) / 128, 128, 0, st>>>(a);
             hp_count_launch();
             if (b == 12 && !getenv("HP_SETUP_THREAD")) hp_sep_chain_half_kernel<12><<<(a.nb * 2 + 7) / 8, 128, 0, st>>>(a);
             else if (small_b) hp_sep_chain_kernel<144><<<(a.nb * 2 + 31) / 32, 32, 0, st>>>(a); else hp_sep_chain_kernel<HP_BMAX * HP_BMAX><<<(a.nb * 2 + 31) / 32, 32, 0, st>>>(a);

@@ -27,11 +27,12 @@ struct HpStripCtx {
     const cplx* s1t;      // s1 on the x1 half grid, t = 0..2n+2
     const cplx* is1t;     // 1/s1
     const double* c_mat;  // (n+2) x (n+2), row major, indexed [i-1][j-1] as the reference does
+    const cplx* kappa_c = nullptr;   // attenuating medium: n x n complex slowness^2, grid aligned (hp_block_row<true>)
 };
 
 // Forward Schur chain of one leaf: Finv[i] = (D_i - L_i Finv[i-1] U_{i-1})^{-1}, i = i0..i1 (1-based,
 // inclusive).  out points at this strip's [n][b*b] scratch.
-template <int BB = HP_BMAX * HP_BMAX>
+template <int BB = HP_BMAX * HP_BMAX, bool CK = false>
 HP_HD int hp_chain_forward(cplx* out, int i0, int i1, int m, const HpStripCtx& c) {
     const int b = c.b, bb = b * b;
     HpStripRow R;
@@ -41,7 +42,7 @@ HP_HD int hp_chain_forward(cplx* out, int i0, int i1, int m, const HpStripCtx& c
     cplx F[BB];
     int bad = 0;
     for (int i = i0; i <= i1; ++i) {
-        hp_block_row(B, R, i, m, b, c.n, c.pml, c.s1t, c.is1t, c.c_mat, c.omega2);
+        hp_block_row<CK>(B, R, i, m, b, c.n, c.pml, c.s1t, c.is1t, c.c_mat, c.omega2, c.kappa_c);
         hp_schur_step(F, B, B.L, i > i0 ? out + (size_t)(i - 2) * bb : out, Uprev, b, i > i0);
         bad |= hp_inv_inplace(F, b);
         cplx* dst = out + (size_t)(i - 1) * bb;
@@ -55,7 +56,7 @@ HP_HD int hp_chain_forward(cplx* out, int i0, int i1, int m, const HpStripCtx& c
 // ascending recurrence for the diagonal blocks of the leaf inverse
 //   G_{i0,i0} = Binv[i0],   G_ii = Binv_i + Binv_i L_i G_{i-1,i-1} U_{i-1} Binv_i
 // of which only the last column (source in the last strip row) is kept: gcol[i][0..b).
-template <int BB = HP_BMAX * HP_BMAX>
+template <int BB = HP_BMAX * HP_BMAX, bool CK = false>
 HP_HD int hp_chain_backward(cplx* out, cplx* gcol, int i0, int i1, int m, const HpStripCtx& c) {
     const int b = c.b, bb = b * b;
     HpStripRow R;
@@ -65,7 +66,7 @@ HP_HD int hp_chain_backward(cplx* out, cplx* gcol, int i0, int i1, int m, const 
     cplx F[BB];
     int bad = 0;
     for (int i = i1; i >= i0; --i) {
-        hp_block_row(B, R, i, m, b, c.n, c.pml, c.s1t, c.is1t, c.c_mat, c.omega2);
+        hp_block_row<CK>(B, R, i, m, b, c.n, c.pml, c.s1t, c.is1t, c.c_mat, c.omega2, c.kappa_c);
         hp_schur_step(F, B, B.U, i < i1 ? out + (size_t)i * bb : out, Lnext, b, i < i1);
         bad |= hp_inv_inplace(F, b);
         cplx* dst = out + (size_t)(i - 1) * bb;
@@ -80,7 +81,7 @@ HP_HD int hp_chain_backward(cplx* out, cplx* gcol, int i0, int i1, int m, const 
     cplx Uprev[HP_BMAX];
     for (int i = i0; i <= i1; ++i) {
         const cplx* Bi = out + (size_t)(i - 1) * bb;
-        hp_block_row(B, R, i, m, b, c.n, c.pml, c.s1t, c.is1t, c.c_mat, c.omega2);
+        hp_block_row<CK>(B, R, i, m, b, c.n, c.pml, c.s1t, c.is1t, c.c_mat, c.omega2, c.kappa_c);
         if (i == i0) {
             for (int e = 0; e < bb; ++e) G[e] = Bi[e];
         } else {
@@ -181,12 +182,13 @@ HP_HD void hp_leaf_corner_tp(cplx* out, const cplx* Binv, int i0, int q, int qlo
 //   S_jj     = D_s - L_s tt_left U_{s-1} - U_s pp_right L_{s+1}
 //   S_j,j+1  = -U_s pt U_t           with pt = tp^T of the leaf between separators j and j+1 (t = s'-1)
 // ---------------------------------------------------------------------------------------------
+template <bool CK = false>
 HP_HD void hp_sep_diag(cplx* S, int s, int m, const cplx* tt_left, const cplx* pp_right, const HpStripCtx& c) {
     const int b = c.b;
     HpStripRow R;
     hp_strip_rows(R, m, b, c.pml);
     HpBlockRow B;
-    hp_block_row(B, R, s, m, b, c.n, c.pml, c.s1t, c.is1t, c.c_mat, c.omega2);
+    hp_block_row<CK>(B, R, s, m, b, c.n, c.pml, c.s1t, c.is1t, c.c_mat, c.omega2, c.kappa_c);
     for (int r = 0; r < b; ++r)
         for (int t = 0; t < b; ++t) {
             cplx v = cmake(0.0, 0.0);

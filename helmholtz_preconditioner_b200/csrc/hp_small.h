@@ -34,6 +34,16 @@ HP_HD cplx cfma(cplx a, cplx b, cplx c) {
 HP_HD cplx cfms(cplx a, cplx b, cplx c) {
     return cmake(fma(a.y, b.y, fma(-a.x, b.x, c.x)), fma(-a.y, b.x, fma(-a.x, b.y, c.y)));
 }
+// kappa * z for the slowness^2 of a real (double) or an attenuating (complex) medium.  With a zero imaginary part the
+// complex product gives the bits of the real scaling: k*z.x - 0*z.y and k*z.y + 0*z.x round like k*z.x and k*z.y.
+HP_HD cplx hp_kmul(double k, cplx z) { return cscale(k, z); }
+HP_HD cplx hp_kmul(cplx k, cplx z) { return cmul(k, z); }
+// kappa * z - s, the diagonal coefficient c5.  The real medium's k*z.x - s.x compiles to one fma (the product is not
+// rounded), so cmul(kappa, z) - s would round differently even for Im(kappa) = 0.  The complex form is therefore
+// Re(kappa) z - s + Im(kappa) (i z): its first part is the real medium's expression, and a zero imaginary part adds
+// exact zeros, which keeps the bits of the real medium.
+HP_HD cplx hp_kmul_sub(double k, cplx z, cplx s) { return csub(cscale(k, z), s); }
+HP_HD cplx hp_kmul_sub(cplx k, cplx z, cplx s) { return cadd(csub(cscale(k.x, z), s), cscale(k.y, cmake(-z.y, z.x))); }
 HP_HD double cabs2(cplx a) { return a.x * a.x + a.y * a.y; }
 // Smith's algorithm, the same scheme CPython / numpy use for complex division
 HP_HD cplx cdiv(cplx a, cplx b) {
@@ -178,12 +188,16 @@ HP_HD void hp_strip_rows(HpStripRow& R, int m, int b, const HpPml& p) {
 //   c3 = 1/h^2 * s2m((j-.5)h)/s1(ih)      -> sub[k]   (coupling to k-1)
 //   c4 = 1/h^2 * s2m((j+.5)h)/s1(ih)      -> sup[k]   (coupling to k+1)
 //   c5 = omega^2/(s1 s2m c^2) - (c1+c2+c3+c4)
+// CK selects the medium: false reads the real velocity c_mat, true the complex slowness^2 kappa_c of an attenuating medium
+// (grid aligned, kappa_c[(j-1) n + (i-1)] = 1/c_mat[i-1][j-1]^2, see hp_kappa_c_kernel).  The complex c5 is formed by
+// hp_kmul_sub, so that a zero imaginary part gives the bits of the real medium.
 struct HpBlockRow {
     cplx L[HP_BMAX], U[HP_BMAX], sub[HP_BMAX], dia[HP_BMAX], sup[HP_BMAX];
 };
 
+template <bool CK = false>
 HP_HD void hp_block_row(HpBlockRow& B, const HpStripRow& R, int i, int m, int b, int n, const HpPml& p,
-                        const cplx* s1t, const cplx* is1t, const double* c_mat, cplx omega2) {
+                        const cplx* s1t, const cplx* is1t, const double* c_mat, cplx omega2, const cplx* kappa_c = nullptr) {
     double ih2 = 1.0 / (p.h * p.h);
     cplx s1lo = s1t[2 * i - 1], s1hi = s1t[2 * i + 1], is1c = is1t[2 * i];
     for (int k = 0; k < b; ++k) {
@@ -192,9 +206,15 @@ HP_HD void hp_block_row(HpBlockRow& B, const HpStripRow& R, int i, int m, int b,
         cplx c2 = cscale(ih2, cmul(s1hi, R.is2c[k]));
         cplx c3 = cscale(ih2, cmul(R.s2lo[k], is1c));
         cplx c4 = cscale(ih2, cmul(R.s2hi[k], is1c));
-        double cv = c_mat[(size_t)(i - 1) * (n + 2) + (j - 1)];          // c_mat[i-1, j-1], code.py:270
-        cplx c5 = cscale(1.0 / (cv * cv), cmul(omega2, cmul(is1c, R.is2c[k])));
-        c5 = csub(c5, cadd(cadd(c1, c2), cadd(c3, c4)));
+        cplx c5;
+        if (CK) {
+            c5 = hp_kmul_sub(kappa_c[(size_t)(j - 1) * n + (i - 1)], cmul(omega2, cmul(is1c, R.is2c[k])),
+                             cadd(cadd(c1, c2), cadd(c3, c4)));
+        } else {
+            double cv = c_mat[(size_t)(i - 1) * (n + 2) + (j - 1)];      // c_mat[i-1, j-1], code.py:270
+            c5 = cscale(1.0 / (cv * cv), cmul(omega2, cmul(is1c, R.is2c[k])));
+            c5 = csub(c5, cadd(cadd(c1, c2), cadd(c3, c4)));
+        }
         B.L[k] = c1; B.U[k] = c2; B.sub[k] = c3; B.sup[k] = c4; B.dia[k] = c5;
     }
 }

@@ -74,3 +74,18 @@ def init_layered_f1(omega, n, layers=8, c_lo=1.0, c_hi=2.0, fr1=.5, fr2=.125, se
     prof[prof < c_lo * 0.5] = c_lo
     c_mat = np.tile(prof[None, :], (n + 2, 1))     # varies with the second index = x2 (depth)
     return c_mat, init_f1_mat(fr1, fr2, omega, n)
+
+
+def attenuate(c_mat, q):
+    """Attenuating medium from a velocity model and a quality factor: returns c_mat / sqrt(1 + 1j/q), complex.
+
+    q is a scalar or an array of c_mat's shape; np.inf means lossless (the result then has a zero imaginary part).
+    Sign convention: the solver's PML, s = 1/(1 + i sigma/omega), and a damping alpha > 0 in
+    omega = 2 pi wave_num + 1j alpha both make loss Im(omega^2 kappa) > 0 for Re omega > 0, with the slowness^2
+    kappa = 1/c^2.  Here kappa = (1 + 1j/q)/c_mat^2, so Im(kappa) > 0 for 0 < q < inf: a wave decays as it travels.
+    Pass the result as c_mat to HelmholtzSolver, run_solver, run_solver_many or any other entry point."""
+    c = np.asarray(c_mat)
+    q = np.asarray(q, dtype=np.float64)
+    if q.ndim and q.shape != c.shape:
+        raise ValueError(f"q must be a scalar or of c_mat's shape {c.shape}, got {q.shape}")
+    return c / np.sqrt(1 + 1j / q)

@@ -42,13 +42,25 @@ def _as_device_field(x, device):
     return torch.from_numpy(a).to(device)
 
 
+def _is_complex_medium(c_mat):
+    """True for a velocity model of complex dtype (an attenuating medium), judged by the dtype alone."""
+    if isinstance(c_mat, torch.Tensor):
+        return c_mat.is_complex()
+    return np.iscomplexobj(c_mat)
+
+
 class HelmholtzSolver:
     """One problem instance on one device: owns the hp_solver handle (tables, velocity, factorisation).
 
     Arguments are the reference's: n interior points per side, b PML width in points, omega complex angular
-    frequency (2*pi*wave_num + 1j*alpha, code.py:442), const the PML strength, c_mat the (n+2)^2 velocity."""
+    frequency (2*pi*wave_num + 1j*alpha, code.py:442), const the PML strength, c_mat the (n+2)^2 velocity.
+    A c_mat of complex dtype (numpy, or a torch tensor on the host or the device) is an attenuating medium
+    (hp_create_complex, see fields.attenuate); a real dtype gives the lossless path."""
 
     def __init__(self, n, b, omega, const, c_mat, device=None):
+        cplx_medium = _is_complex_medium(c_mat)
+        if cplx_medium and tuple(c_mat.shape) != (n + 2, n + 2):
+            raise ValueError(f"c_mat must be ({n + 2}, {n + 2}) like the reference's init_c*_mat, got {tuple(c_mat.shape)}")
         self.lib = _lib.require_device()
         self.device = torch.device(device if device is not None else f"cuda:{torch.cuda.current_device()}")
         if self.device.index is None:
@@ -56,7 +68,17 @@ class HelmholtzSolver:
         self.n, self.b, self.omega, self.const = int(n), int(b), complex(omega), float(const)
         self.h = 1 / (n + 1)
         self.eta = b * self.h
-        if isinstance(c_mat, torch.Tensor) and c_mat.is_cuda:
+        create = self.lib.hp_create
+        if cplx_medium:
+            create = self.lib.hp_create_complex
+            if isinstance(c_mat, torch.Tensor) and c_mat.is_cuda:
+                c_dev = c_mat.to(dtype=torch.complex128).contiguous()
+                cptr, on_dev = c_dev.data_ptr(), 1
+            else:
+                c_np = c_mat.detach().resolve_conj().numpy() if isinstance(c_mat, torch.Tensor) else c_mat
+                c_host = np.ascontiguousarray(np.asarray(c_np, dtype=np.complex128))
+                cptr, on_dev = c_host.ctypes.data, 0
+        elif isinstance(c_mat, torch.Tensor) and c_mat.is_cuda:
             c_dev = c_mat.to(dtype=torch.float64).contiguous()
             cptr, on_dev = c_dev.data_ptr(), 1
         else:
@@ -66,12 +88,18 @@ class HelmholtzSolver:
         if shape != (n + 2, n + 2):
             raise ValueError(f"c_mat must be ({n + 2}, {n + 2}) like the reference's init_c*_mat, got {shape}")
         h = C.c_void_p()
+        what = "hp_create_complex" if cplx_medium else "hp_create"
         with torch.cuda.device(self.device):
-            _lib.check(self.lib.hp_create(C.byref(h), self.n, self.b, self.omega.real, self.omega.imag, self.const,
-                                          cptr, on_dev, _stream()), "hp_create")
+            _lib.check(create(C.byref(h), self.n, self.b, self.omega.real, self.omega.imag, self.const,
+                              cptr, on_dev, _stream()), what)
         self.handle = h
         self.m_lo, self.m_hi = 0, -1
         self.max_group = 8            # cap on the right-hand sides per sweep launch (1 = one launch per vector)
+
+    @property
+    def medium_is_complex(self):
+        """True when the solver holds an attenuating (complex) medium, made from a c_mat of complex dtype."""
+        return bool(self.lib.hp_medium_is_complex(self.handle))
 
     def clone_context(self):
         """A second handle on this solver's operator and factorisation with private sweep scratch (hp_context_clone):

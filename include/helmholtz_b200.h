@@ -39,6 +39,17 @@ int hp_profile_read(hp_solver* s, double* sweep_ms, int* launches, int64_t* byte
  * c_is_device != 0 means c_mat already lives on the device. */
 int hp_create(hp_solver** out, int n, int b, double omega_re, double omega_im, double cst,
               const double* c_mat, int c_is_device, void* stream);
+/* Attenuating medium: the same problem with a complex velocity.  c_mat holds (n+2) x (n+2) complex numbers, interleaved
+ * (real, imaginary) doubles in the same row-major order.  The solver keeps only the complex slowness^2
+ * kappa = 1/c^2 on the grid (16 B per point) and every function below reads it: hp_assemble_csr, hp_assemble_strip_csr,
+ * hp_stencil_matvec(_rows), hp_precond_setup with both front blocks, and everything that applies the preconditioner.
+ * Loss means Im(omega^2 kappa) > 0 for Re omega > 0, the sign of the PML and of alpha > 0.  A velocity with zero
+ * imaginary parts gives the bits of hp_create.  The setup generations selected by the developer switches
+ * HP_CHAIN_THREAD and HP_CHAIN_UNROLL refuse a complex medium. */
+int hp_create_complex(hp_solver** out, int n, int b, double omega_re, double omega_im, double cst,
+                      const double* c_mat, int c_is_device, void* stream);
+/* 1 if the solver (or the solver a context was cloned from) was made by hp_create_complex, 0 if by hp_create */
+int hp_medium_is_complex(hp_solver* s);
 int hp_destroy(hp_solver* s);
 /* A second handle on a solver that is set up: shares the operator tables and the factorisation (read-only) and owns a
  * private copy of the sweep scratch (exchange ring, abort flags, parked front solutions T_F u_F of code.py:364), so that

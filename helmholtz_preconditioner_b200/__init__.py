@@ -11,6 +11,9 @@ def __getattr__(name):
     if name in ("HelmholtzSolver", "DeviceCSR", "SolveResult", "run_solver", "run_solver_many", "build_A_matrix", "algo2_3", "algo2_4", "get_Hm", "get_A_FF_block"):
         from . import solver
         return getattr(solver, name)
+    if name in ("Receivers", "GradientResult", "misfit_gradient", "born"):
+        from . import inversion
+        return getattr(inversion, name)
     if name in ("gmres", "gmres_batch", "DeviceVectors", "lartg"):
         import importlib
         return getattr(importlib.import_module(__name__ + ".gmres"), name)

@@ -65,6 +65,9 @@ SIGNATURES = {
     "hp_strip_apply": (_i, [_vp, _i, _vp, _vp, _vp]),
     "hp_strip_layout": (_i, [_vp, _ip, _ip, _ip, _ip, _ip, _ip, C.POINTER(_i64), _ip, _ip, _ip]),
     "hp_strip_packets": (_i, [_vp, _i, _vp]),
+    "hp_grad_accumulate": (_i, [_vp, _i, C.POINTER(_vp), C.POINTER(_vp), _vp, _vp]),
+    "hp_grad_finish": (_i, [_vp, _vp, _i, _vp, _vp]),
+    "hp_born_source": (_i, [_vp, _i, _vp, C.POINTER(_vp), C.POINTER(_vp), _vp]),
     "hp_dotc": (_i, [_i64, _vp, _vp, _vp, _vp]),
     "hp_nrm2": (_i, [_i64, _vp, _vp, _vp]),
     "hp_axpy": (_i, [_i64, _d, _d, _vp, _vp, _vp]),

@@ -6,7 +6,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libhelmholtz_b200.so")
-SOURCES = ["hp_api.cu", "hp_assembly.cu", "hp_blas.cu", "hp_setup.cu", "hp_front.cu", "hp_front_coupled.cu", "hp_sweep.cu", "hp_sweep2.cu", "hp_sweep4.cu", "hp_sweep4m.cu", "hp_sweep4d.cu", "hp_peer.cu", "hp_cgs.cu"]
+SOURCES = ["hp_api.cu", "hp_assembly.cu", "hp_blas.cu", "hp_setup.cu", "hp_front.cu", "hp_front_coupled.cu", "hp_sweep.cu", "hp_sweep2.cu", "hp_sweep4.cu", "hp_sweep4m.cu", "hp_sweep4d.cu", "hp_peer.cu", "hp_cgs.cu", "hp_grad.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "--fmad=true"]
 

@@ -537,6 +537,32 @@ def _source_fields(f_mats, n, device):
     return fs
 
 
+def _solve_wave(s, wave, W, vec, diag, precond_input, rtol, restart, maxiter):
+    """One wave of at most W = s._widest() sources (device fields) by batched GMRES, source i pinned to slot i of every
+    sweep launch, converged or idle slots left empty.  Returns gmres_batch's [(u, info, hist)] after checking the sweep
+    status.  Shared by run_solver_many and the inversion drivers (inversion.py)."""
+    Mf = None
+    if precond_input == "rhs":
+        # as in run_solver, M f is computed once and copied: one launch for the whole wave
+        Mf = [torch.empty_like(f) for f in wave]
+        s.precond_apply_slots([(f, m) for f, m in zip(wave, Mf)] + [None] * (W - len(wave)), diag=diag)
+
+    def psolve_batch(reqs):
+        if Mf is not None:
+            for i, _, out in reqs:
+                vec.scale_copy(1.0, Mf[i], out)
+            return
+        slots = [None] * W
+        for i, x, out in reqs:
+            slots[i] = (x, out)
+        s.precond_apply_slots(slots, diag=diag)
+
+    outs = gmres_batch(lambda x, out: s.matvec(x, out), psolve_batch, wave, vec=vec, with_index=True, rtol=rtol,
+                       restart=restart, maxiter=maxiter, health=s.check_status)
+    s.check_status()
+    return outs
+
+
 def run_solver_many(n, b, wave_num, const, alpha, f_mats, init_func=fields.init_c1_f1, *, c_mat=None, diag="reference",
                     precond_input="rhs", front="blockdiag", rtol=1e-3, restart=20, maxiter=None, device=None, P=0, K=0,
                     verbose=True, solver=None):
@@ -569,26 +595,7 @@ def run_solver_many(n, b, wave_num, const, alpha, f_mats, init_func=fields.init_
     results = []
     for w0 in range(0, len(fs), W):
         tw = time.time()
-        wave = fs[w0:w0 + W]
-        Mf = None
-        if precond_input == "rhs":
-            # as in run_solver, M f is computed once and copied: one launch for the whole wave
-            Mf = [torch.empty_like(f) for f in wave]
-            s.precond_apply_slots([(f, m) for f, m in zip(wave, Mf)] + [None] * (W - len(wave)), diag=diag)
-
-        def psolve_batch(reqs, Mf=Mf):
-            if Mf is not None:
-                for i, _, out in reqs:
-                    vec.scale_copy(1.0, Mf[i], out)
-                return
-            slots = [None] * W
-            for i, x, out in reqs:
-                slots[i] = (x, out)
-            s.precond_apply_slots(slots, diag=diag)
-
-        outs = gmres_batch(lambda x, out: s.matvec(x, out), psolve_batch, wave, vec=vec, with_index=True, rtol=rtol,
-                           restart=restart, maxiter=maxiter, health=s.check_status)
-        s.check_status()
+        outs = _solve_wave(s, fs[w0:w0 + W], W, vec, diag, precond_input, rtol, restart, maxiter)
         t_wave = time.time() - tw
         for j, (u, info, hist) in enumerate(outs):
             results.append(SolveResult(u, hist, len(hist), info, t1 - t0, t_wave, s))

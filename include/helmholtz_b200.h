@@ -155,6 +155,25 @@ int hp_strip_packets(hp_solver* s, int m, double* packets_host);
  * right-hand sides, rows of x and gathered entries per CTA */
 int hp_strip_layout_ex(hp_solver* s, int* colN, int* NCB, int* NRQ, int* NXG);
 
+/* ---- inversion (helmholtz_preconditioner_b200/inversion.py) -----------------------------------------
+ * The reference has no counterpart.  With w_p = omega^2 is1(i) is2(j) = dA_pp/dkappa_p (the factor the diagonal c5
+ * multiplies the slowness^2 kappa = 1/c^2 by), fields u (A u = f) and adjoint fields mu (A mu = R^T conj(r); A is complex
+ * symmetric) in the vector layout above, the misfit gradient is G = -conj(w (.) sum_s mu_s (.) u_s) and the Born source
+ * of a perturbation dkappa is -w (.) dkappa (.) u.  u_devs / mu_devs / out_devs are HOST arrays of R device pointers,
+ * 1 <= R <= 8; a slot whose two pointers are NULL is skipped, a slot with one NULL pointer is refused, and at least one
+ * slot must be active.  Each result is deterministic. */
+/* acc_dev[p] += u_r[p] mu_r[p] for the active slots in the order r = 0..R-1 (n*n complex accumulator) */
+int hp_grad_accumulate(hp_solver* s, int R, const double* const* u_devs, const double* const* mu_devs, double* acc_dev,
+                       void* stream);
+/* G = -conj(w (.) acc); wrt = 1 multiplies by conj(dkappa/dc) = conj(-2 kappa sqrt(kappa)) (principal root).  Written in
+ * the c_mat layout: out_dev[(i-1)(n+2) + (j-1)] belongs to grid point (i, j), the last two rows and columns are zero.
+ * (n+2)^2 float64 (Re G) for a medium made by hp_create, complex128 for one made by hp_create_complex. */
+int hp_grad_finish(hp_solver* s, const double* acc_dev, int wrt, double* out_dev, void* stream);
+/* out_r = -w (.) dkappa (.) u_r for the active slots; dkappa_dev is (n+2)^2 complex128 in the c_mat layout (entry
+ * [i-1][j-1] for grid point (i, j); the last two rows and columns are not read).  out_devs[r] may equal u_devs[r]. */
+int hp_born_source(hp_solver* s, int R, const double* dkappa_dev, const double* const* u_devs, double* const* out_devs,
+                   void* stream);
+
 /* ---- Krylov vector kernels (scipy gmres inner loop, iterative.py; called from code.py:516) -------- */
 
 /* out_dev[0..1] = sum conj(x) y   (np.vdot) */

@@ -71,6 +71,19 @@ __device__ __forceinline__ cplx cfrag_get4(const CFrag (&c)[NST], int i) {
 }
 __device__ __forceinline__ cplx cz() { return cmake(0.0, 0.0); }
 
+// State of the separator column b-1 carried from strip to strip for two right-hand sides, one per lane that owns it
+// (4 lanes of critical warp 0).  It lives in shared memory: held in registers, it pushed the critical warps past the
+// 168-register cap and the whole per-strip loop spilled to local memory.
+struct HpSepState { cplx usbase[2], vsb[2], o_usep[2], o_usbase[2], o_c, cis1, ys[2], usep[2]; };
+// u[i] -> shared memory without a register (cp.async, waited for with cp_async_wait_all); a masked slot (u = NULL) or
+// take = false gives 0 and reads nothing (src-size 0; `any` is only a valid address)
+__device__ __forceinline__ void cp_async_slot(cplx* dst, const cplx* u, size_t i, bool take, const void* any) {
+    const bool rd = take && u;
+    asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(smem_u32(dst)), "l"(rd ? (const void*)(u + i) : any),
+                 "r"(rd ? 16 : 0) : "memory");
+}
+__device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
+
 // MODE: 0 forward, 1 backward (reference diagonal), 2 backward (paper diagonal)
 template <int MODE, bool DBG, int BT, int KT>
 __global__ void __launch_bounds__(HP4D_THREADS, 1) hp_sweep4d_kernel(HpSweepArgs a, Hp4dPlan pl) {
@@ -109,7 +122,8 @@ __global__ void __launch_bounds__(HP4D_THREADS, 1) hp_sweep4d_kernel(HpSweepArgs
     cplx* glp = x3 + 2 * (size_t)RT * B3V;                       // [2][K][b][RT]      (DSMEM target)
     cplx* rho_p = glp + 2 * (size_t)K * b * RT;                  // [3][RT][BV]        partial sums of -rho (one per critical warp)
     cplx* gfp = rho_p + 3 * (size_t)RT * BV;                     // [2][b][RT]         gf partials of leaf l+1, summed over its K parts
-    unsigned long long* mbar = reinterpret_cast<unsigned long long*>(gfp + 2 * (size_t)b * RT);
+    HpSepState* sep_st = reinterpret_cast<HpSepState*>(gfp + 2 * (size_t)b * RT);   // [4]   one per lane ft of the separator column
+    unsigned long long* mbar = reinterpret_cast<unsigned long long*>(sep_st + 4);
     unsigned long long* barW = mbar;                 // [S]
     unsigned long long* barG = barW + S;             // [3]
     unsigned long long* barN = barG + 3;             // [2]
@@ -164,28 +178,26 @@ __global__ void __launch_bounds__(HP4D_THREADS, 1) hp_sweep4d_kernel(HpSweepArgs
         const int sep_tile = (b - 1) >> 3;
         const bool is_sep = has_sep && cw == 0 && fg == ((b - 1) & 7);
         const int sep_col = has_sep ? a.sep[l] : 0;
-        cplx* const u0 = a.um[2 * ft];
-        cplx* const u1 = a.um[2 * ft + 1];
-        const cplx cis1s = is_sep ? a.is1t[2 * (sep_col + 1)] : cz();
-        cplx usbase[2] = {cz(), cz()}, vsb[2] = {cz(), cz()}, o_usep[2] = {cz(), cz()}, o_usbase[2] = {cz(), cz()};
-        cplx o_c = cz();
+        HpSepState& ss = sep_st[ft];                  // zero from the fill above; touched by the is_sep lanes only
         if (is_sep) {
+            const cplx cis1s = a.is1t[2 * (sep_col + 1)];
+            ss.cis1 = cis1s;
 #pragma unroll
             for (int i = 0; i < 2; ++i) {
-                cplx* u = i ? u1 : u0;
-                if (a_mode == 0) vsb[i] = ldcg_slot(u, (size_t)(m0 - 1) * n + sep_col);
+                cplx* u = a.um[2 * ft + i];
+                if (a_mode == 0) ss.vsb[i] = ldcg_slot(u, (size_t)(m0 - 1) * n + sep_col);
                 else {
-                    usbase[i] = ldcg_slot(u, (size_t)(m0 - 1) * n + sep_col);
-                    vsb[i] = usbase[i];
-                    if (m0 < n) vsb[i] = cfma(cscale(sg, cmul(hp_rowfac(a, m0), cis1s)), ldcg_slot(u, (size_t)m0 * n + sep_col), vsb[i]);
+                    const cplx ub = ldcg_slot(u, (size_t)(m0 - 1) * n + sep_col);
+                    ss.usbase[i] = ub;
+                    ss.vsb[i] = m0 < n ? cfma(cscale(sg, cmul(hp_rowfac(a, m0), cis1s)), ldcg_slot(u, (size_t)m0 * n + sep_col), ub) : ub;
                 }
             }
         }
         auto sep_output = [&](int m_prev, int i, cplx ys) {   // y_s = x_l[b-1] of strip m_prev, right-hand side 2 ft + i
             if (k != 0) return;
-            cplx* u = i ? u1 : u0;
-            if (a_mode == 0) st_slot(u, (size_t)m_prev * n + sep_col, cfms(o_c, ys, o_usep[i]));
-            else st_slot(u, (size_t)(m_prev - 1) * n + sep_col, a_diag == 0 ? csub(o_usbase[i], ys) : ys);
+            cplx* u = a.um[2 * ft + i];
+            if (a_mode == 0) st_slot(u, (size_t)m_prev * n + sep_col, cfms(ss.o_c, ys, ss.o_usep[i]));
+            else st_slot(u, (size_t)(m_prev - 1) * n + sep_col, a_diag == 0 ? csub(ss.o_usbase[i], ys) : ys);
         };
         const int nks_b = (b3 + 3) >> 2, ks_per = (nks_b + HP4_CW - 1) / HP4_CW;       // k-steps of P = R X3, split over the warps
         const int ntile_e = (b + 7) >> 3;                                              // entry tiles (2 for b = 12)
@@ -199,15 +211,11 @@ __global__ void __launch_bounds__(HP4D_THREADS, 1) hp_sweep4d_kernel(HpSweepArgs
             cplx* slot_next = a.xch + (size_t)((it + 1) & (HP_RING - 1)) * a.slot_stride;
             const cplx* x3p = x3 + (size_t)(par ^ 1) * RT * B3V;                                // x3(it-1), [RT][B3V]
             if (DBG && tid == 0) tprev = clock64();
-            cplx usep[2] = {cz(), cz()}, cs = cz();
-            if (is_sep) {
-                cs = cmul(hp_rowfac(a, a_mode == 1 ? mn : m), cis1s);
+            if (is_sep) {                                   // the field entries of the separator column, used at the end of the strip
 #pragma unroll
-                for (int i = 0; i < 2; ++i) {
-                    cplx* u = i ? u1 : u0;
-                    if (a_mode == 0) usep[i] = ldcg_slot(u, (size_t)m * n + sep_col);
-                    else if (more) usep[i] = ldcg_slot(u, (size_t)(mn - 1) * n + sep_col);
-                }
+                for (int i = 0; i < 2; ++i)
+                    cp_async_slot(&ss.usep[i], a.um[2 * ft + i], a_mode == 0 ? (size_t)m * n + sep_col : (size_t)(mn - 1) * n + sep_col,
+                                  a_mode == 0 || more, a.is1t);
             }
             // ---- x-independent part: the K partial sums of gl (DSMEM) and gf (L2, poll warp), split over the warps
             CFrag acc[2][2];                                // entry tiles 0, 1 (b <= 16: see the host check), two k-streams each
@@ -264,21 +272,15 @@ __global__ void __launch_bounds__(HP4D_THREADS, 1) hp_sweep4d_kernel(HpSweepArgs
                     const int e = fg + 8 * t;
                     if (t < ntile_e && e < b) {
                         cplx r0 = cadd(acc[t][0].get(0), acc[t][1].get(0)), r1 = cadd(acc[t][0].get(1), acc[t][1].get(1));
-                        if (is_sep && t == sep_tile) { r0 = csub(r0, vsb[0]); r1 = csub(r1, vsb[1]); }
+                        if (is_sep && t == sep_tile) { r0 = csub(r0, ss.vsb[0]); r1 = csub(r1, ss.vsb[1]); }
                         rho_p[((size_t)cw * RT + 2 * ft) * BV + e] = r0;
                         rho_p[((size_t)cw * RT + 2 * ft + 1) * BV + e] = r1;
                     }
                 }
             }
-            if (is_sep) {
-#pragma unroll
-                for (int i = 0; i < 2; ++i) {
-                    if (it > 0) sep_output(m - step, i, x3p[(size_t)(2 * ft + i) * B3V + b2 - 1]);
-                    o_usep[i] = usep[i]; o_usbase[i] = usbase[i];
-                    if (a_mode == 0) vsb[i] = usep[i];
-                    else { vsb[i] = a_diag == 0 ? cfma(cs, usbase[i], usep[i]) : usep[i]; usbase[i] = usep[i]; }
-                }
-                o_c = cs;
+            if (is_sep && it > 0) {
+                ss.ys[0] = x3p[(size_t)(2 * ft) * B3V + b2 - 1];     // x3(it-1) is overwritten from strip it+1 on
+                ss.ys[1] = x3p[(size_t)(2 * ft + 1) * B3V + b2 - 1];
             }
             if (has_sep) {
                 bar_crit4();
@@ -330,7 +332,9 @@ __global__ void __launch_bounds__(HP4D_THREADS, 1) hp_sweep4d_kernel(HpSweepArgs
                 if (lane == 0) { mbar_arrive_local(&eN[par]); mbar_arrive_local(&eR[par]); }
                 if (ctid == 0 && it + 2 < nsteps) mbar_expect_tx(&barGL[par], gl_bytes);
             }
-            // ---- D: gather x3(it): a warp load covers 4 separators x 8 right-hand sides of one entry
+            // ---- D: gather x3(it): a warp load covers 4 separators x 8 right-hand sides of one entry.  The separator column's
+            //      field reads of this strip complete before it: x3(it) lets the CTA k = 0 of the leaf overwrite that entry.
+            if (is_sep) cp_async_wait_all();
             if (any_sep) {
                 const int lr = lane % RT, lsub = lane / RT;
                 constexpr int SPL = 32 / RT;
@@ -389,6 +393,20 @@ __global__ void __launch_bounds__(HP4D_THREADS, 1) hp_sweep4d_kernel(HpSweepArgs
                     }
                 }
                 HPD_TICK(5);
+            }
+            // ---- the separator column: output of strip it-1 and the state of strip it+1, after this strip's hand-over so that
+            //      neither the field load nor the store holds up the critical warps
+            if (is_sep) {
+                const cplx cs = cmul(hp_rowfac(a, a_mode == 1 ? mn : m), ss.cis1);
+#pragma unroll
+                for (int i = 0; i < 2; ++i) {
+                    if (it > 0) sep_output(m - step, i, ss.ys[i]);
+                    const cplx ub = ss.usbase[i], usep = ss.usep[i];
+                    ss.o_usep[i] = usep; ss.o_usbase[i] = ub;
+                    if (a_mode == 0) ss.vsb[i] = usep;
+                    else { ss.vsb[i] = a_diag == 0 ? cfma(cs, ub, usep) : usep; ss.usbase[i] = usep; }
+                }
+                ss.o_c = cs;
             }
         }
         if (any_sep && nsteps > 0 && is_sep) {
@@ -710,7 +728,8 @@ static int hp_sweep4d_plan(const HpLayout& L, int b, size_t max_smem, Hp4dPlan& 
     pl.n_st = al128d(std::max<size_t>(1, (size_t)b * pl.NRQV) * sizeof(cplx));
     pl.r_st = al128d((size_t)b * 3 * b * sizeof(cplx));
     size_t small = sizeof(cplx) * ((size_t)RT * pl.CWV + 2 * (size_t)RT * pl.QPV + 2 * (size_t)RT * pl.CWV + 2 * (size_t)RT * pl.B3V +
-                                   2 * (size_t)L.K * b * RT + 2 * (size_t)b * RT + 3 * (size_t)RT * pl.BV) + 8 * (2 * 8 + 13 + 7 + 4) + 16;
+                                   2 * (size_t)L.K * b * RT + 2 * (size_t)b * RT + 3 * (size_t)RT * pl.BV) + 4 * sizeof(HpSepState) +
+                  8 * (2 * 8 + 13 + 7 + 4) + 16;
     size_t fixed = 3 * pl.g_st + 2 * pl.n_st + 2 * pl.r_st + al128d(small);
     if (fixed + 1024 >= max_smem) return 1;
     size_t avail = max_smem - 1024 - fixed;
